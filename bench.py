@@ -8,6 +8,7 @@ synthetic images, through the C++ batch pipeline of the C-ABI (gseg_pool_run).  
 rank segments its own B images per step (images shard, no data-path collective; weak scaling).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl gseg|reference] [--batch B] [--mode all|headline|tiled|jpeg]
+                  [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  `value` = Mpixel/s with the inputs resident in HBM; `e2e` = the same through the
 C-ABI with pinned HOST buffers (H2D image in, D2H label image out -- in the narrowest lossless label type --
@@ -249,6 +250,29 @@ def roofline_of(agg, peak, peak_src, traffic_table):
                           "dram_frac (ncu DRAM bytes / time / peak) is far below frac and the kernels are L2/latency-bound"}
 
 
+DUMP_LABEL_BYTES = 40 << 20
+
+
+def dump_outputs(out_dir, results, dlab):
+    """--dump-outputs: what the headline's last timed step handed its caller, so that two builds run with the same
+    arguments (hence on the same images) can be compared output for output.  Per image of the batch: component count,
+    level count and label bytes of its gseg_pool_run result.  Device output buffer j holds the label image of the last
+    image i of the batch with i % S == j, in the narrowest lossless type its result names; labels.npy keeps those labels
+    at a fixed seeded sample of pixels (label_pixels.npy, flat indices), sized to keep the whole dump under 64 MB."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    B, (S, h, w) = len(results), tuple(dlab.shape)
+    pix = np.sort(np.random.default_rng(0).choice(h * w, min(h * w, DUMP_LABEL_BYTES // (4 * S)), replace=False))
+    raw = dlab.cpu().numpy().reshape(S, -1)
+    images = [max(range(j, B, S)) for j in range(S)]
+    labels = np.stack([raw[j].view({1: np.uint8, 2: np.uint16, 4: np.int32}[results[i].elem_bytes])[pix]
+                       for j, i in enumerate(images)])
+    np.save(os.path.join(out_dir, "labels.npy"), labels.astype(np.float32))   # exact: labels < h * w < 2^24
+    for name, a in (("n_components", [r.n_components for r in results]), ("n_levels", [r.n_levels for r in results]),
+                    ("label_bytes", [r.elem_bytes for r in results]), ("label_images", images), ("label_pixels", pix)):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
+
+
 _T0 = time.perf_counter()
 
 
@@ -271,7 +295,16 @@ def main():
                          "jpeg: headline + the JPEG-fed entries only")
     ap.add_argument("--tiled-size", type=int, default=32768, help="side of the square image of the tiled run")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the headline's last timed step returned as DIR/<name>.npy (rank 0's images)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "gseg" or args.mode == "tiled":
+            ap.error("--dump-outputs writes the headline's outputs: not with --impl reference or --mode tiled")
+        if args.batch % max(1, min(args.contexts, args.batch)):
+            ap.error("--dump-outputs needs --batch to be a multiple of --contexts (one context per device output buffer)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -344,6 +377,8 @@ def main():
     l0 = pool.launch_count()
     ms_dev = timed(step_dev, args.steps, args.warmup)
     launches = (pool.launch_count() - l0) * args.steps // (args.steps + args.warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res_box["dev"], dlab)
     ms_e2e = timed(step_e2e, args.steps, args.warmup)
     d2h = int(sum(r.out_bytes for r in res_box["e2e"]))
     ms_copy = pool.copy_ceiling(jobs_e2e, res_box["e2e"], reps=3)
@@ -495,10 +530,10 @@ def bench_jpeg_fed(args, gseg, batch, torch, dist, world, pool, himgs, hlab, kw,
 
 
 def _pool_config(args, gseg, torch, dist, rank, world, local_rank, timed, *, name, workload, w, h, n_local, contexts, seeds,
-                 params, out_mode, level, out_entries, caps=0, steps=None, warmup=3, scaling="weak", global_images=None):
+                 params, out_mode, level, out_entries, caps=0, warmup=3, scaling="weak", global_images=None):
     """One BASELINE config through the C++ pool: device-resident `value` and pinned-host `e2e`, like the headline."""
     batch = importlib.import_module(PKG + ".batch")
-    steps = steps or max(2, min(args.steps, 5))
+    steps = args.steps
     pool = batch.Pool(gseg, w, h, device=local_rank, contexts=contexts, max_connectivity=params["connectivity"], caps=caps)
     try:
         seg = pool.segs[0]
@@ -586,7 +621,7 @@ def bench_tiled(args, gseg, torch, dist, rank, world, local_rank, timed):
         torch.cuda.synchronize()
         tiler = tiled.DeviceTiler(seg, dist if world > 1 else None)
         kw = dict(sigma=SIGMA, k=K, min_size=MIN_SIZE, connectivity=4, variant=gseg.FELZ)
-        steps, warmup = max(2, min(args.steps, 5)), 2
+        steps, warmup = args.steps, 2
         box = {}
         phases = {}
 
@@ -637,7 +672,7 @@ def bench_large_roofline(args, gseg, torch, rank, local_rank, peak, peak_src):
         kw = dict(sigma=SIGMA, k=K, min_size=MIN_SIZE, connectivity=CONN, variant=gseg.FELZ)
         seg.segment(img, **kw)
         ts = []
-        for _ in range(3):
+        for _ in range(args.steps):
             torch.cuda.synchronize()
             t0 = time.perf_counter()
             seg.segment(img, **kw)
