@@ -1754,12 +1754,13 @@ extern "C" int gseg_synth(gseg_ctx *ctx, uint8_t *out, int w, int h, uint64_t se
 extern "C" int gseg_sort_pairs_u64(gseg_ctx *ctx, uint64_t *keys, uint32_t *vals, int64_t n, int begin_bit, int end_bit) {
     if (!ctx || !keys || n < 0 || begin_bit < 0 || end_bit > 64 || begin_bit >= end_bit) return GSEG_E_ARG;
     CK(cudaSetDevice(ctx->device));
-    const u64 *before = ctx->sort.keys_alt;
-    const u32 *before_s = ctx->sort.status;
+    // The scratch is reallocated exactly when a capacity grows.  Its addresses are no test: a buffer freed and allocated
+    // again can come back at the same address while another one moved.
+    const size_t cap_n = ctx->sort.cap_n, cap_status = ctx->sort.cap_status;
     cudaError_t e = onesweep_sort_pairs(&ctx->sort, (u64 *)keys, (u32 *)vals, (size_t)n, begin_bit, end_bit, ctx->stream);
     if (e != cudaSuccess) return fail(ctx, GSEG_E_CUDA, "onesweep_sort_pairs", e);
     CK(cudaStreamSynchronize(ctx->stream));
-    if (before != ctx->sort.keys_alt || before_s != ctx->sort.status) CK(upload_dd(ctx)); // a larger sort than any before: the scratch moved
+    if (cap_n != ctx->sort.cap_n || cap_status != ctx->sort.cap_status) CK(upload_dd(ctx)); // a larger sort than any before: the scratch moved
     return GSEG_OK;
 }
 

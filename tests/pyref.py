@@ -61,6 +61,58 @@ def edge_list(planes, conn):
     return es, wts
 
 
+def sobel(planes):
+    """Sobel magnitude of the intensity (r + g + b) * 0.33333334, replicated borders, every op rounded to fp32."""
+    I = F(F(planes[0] + planes[1]) + planes[2]) * F(0.33333334)
+    P = np.pad(I, 1, mode="edge")
+    h, w = I.shape
+
+    def at(dx, dy):                  # I at (x + dx, y + dy), borders replicated
+        return P[1 + dy:1 + dy + h, 1 + dx:1 + dx + w]
+
+    two = F(2.0)
+    r = F(at(1, -1) + two * at(1, 0)) + at(1, 1)
+    l = F(at(-1, -1) + two * at(-1, 0)) + at(-1, 1)
+    d = F(at(-1, 1) + two * at(0, 1)) + at(1, 1)
+    u = F(at(-1, -1) + two * at(0, -1)) + at(1, -1)
+    gx, gy = r - l, d - u
+    return np.sqrt(gx * gx + gy * gy).astype(F)
+
+
+def strength_list(G, conn):
+    """Superpixel edge strength, the mean of the two end pixels' Sobel magnitudes: (edge list as edge_list
+    returns it, weights in edge-index order with +inf where the edge does not exist)."""
+    h, w = G.shape
+    D = 4 if conn == 8 else 2
+    es = []
+    wts = np.full(h * w * D, np.inf, F)
+    for d in range(D):
+        for y in range(h):
+            for x in range(w):
+                xx, yy = x + DXY[d][0], y + DXY[d][1]
+                if 0 <= xx < w and 0 <= yy < h:
+                    p, q = y * w + x, yy * w + xx
+                    wt = F(0.5) * F(G[y, x] + G[yy, xx])
+                    wts[d * h * w + p] = wt
+                    es.append((int(F(wt).view(np.uint32)), d * h * w + p, p, q))
+    return es, wts
+
+
+def colour_sums(planes):
+    """Per-pixel colour in 24.8 fixed point: round half to even of plane * 256 (exact in fp32)."""
+    return np.rint(planes * F(256.0)).astype(np.int64).reshape(3, -1).T
+
+
+def mean_distance_weight(wb, sa, na, sb, nb):
+    """Superpixel weight of an edge of strength bits wb between components with colour sums sa, sb and sizes
+    na, nb: strength * sqrt((dr^2 + dg^2) + db^2), d = f32(sum) / f32(size * 256) per channel.  The sums are
+    exact in float64 (|sum| < 2^53), so F(float(.)) rounds them to fp32 once."""
+    fa, fb = F(na) * F(256.0), F(nb) * F(256.0)
+    dr, dg, db = (F(F(float(sa[c])) / fa) - F(F(float(sb[c])) / fb) for c in range(3))
+    s = F(F(dr * dr) + F(dg * dg)) + F(db * db)
+    return int(F(np.uint32(wb).view(F) * np.sqrt(F(s))).view(np.uint32))
+
+
 def kruskal(es, V, k, min_size):
     parent = list(range(V))
     size = [1] * V
@@ -88,17 +140,22 @@ def kruskal(es, V, k, min_size):
     return np.array([find(i) for i in range(V)], np.int32)
 
 
-def boruvka(es, V, variant, k=0.0, min_size=0, max_rounds=64, max_levels=10 ** 9):
-    """variant 0 FELZ / 1 HIER on the contracted multigraph.  Returns (final labels, [level labels])."""
+def boruvka(es, V, variant, k=0.0, min_size=0, max_rounds=64, max_levels=10 ** 9, planes=None):
+    """variant 0 FELZ / 1 HIER / 2 SUPERPIX on the contracted multigraph.  Returns (final labels, [level labels]).
+    SUPERPIX: es carries the static strengths and planes the blurred colour; every round re-weights each edge
+    from the current components' colour sums."""
     label = list(range(V))                      # pixel -> component id (arbitrary ints)
     size = {c: 1 for c in range(V)}
     Int = {c: F(0.0) for c in range(V)}
+    csum = {c: s for c, s in enumerate(colour_sums(planes))} if variant == 2 else None
     medges = [(wb, idx, p, q) for wb, idx, p, q in es]   # (key..., endpoints as component ids)
     phase, levels, out_levels = 0, 0, []
     for _ in range(max_rounds):
         medges = [(wb, idx, a, b) for wb, idx, a, b in medges if a != b]
         best = {}
         for wb, idx, a, b in medges:
+            if variant == 2:
+                wb = mean_distance_weight(wb, csum[a], size[a], csum[b], size[b])
             for c in (a, b):
                 if c not in best or (wb, idx) < best[c][:2]:
                     best[c] = (wb, idx, a, b)
@@ -137,7 +194,7 @@ def boruvka(es, V, variant, k=0.0, min_size=0, max_rounds=64, max_levels=10 ** 9
             return c
 
         rt = {c: root(c) for c in size}
-        nsize, nInt = {}, {}
+        nsize, nInt, nsum = {}, {}, {}
         for c in size:
             r = rt[c]
             nsize[r] = nsize.get(r, 0) + size[c]
@@ -145,7 +202,11 @@ def boruvka(es, V, variant, k=0.0, min_size=0, max_rounds=64, max_levels=10 ** 9
             if succ[c] != c:
                 m = max(m, np.uint32(best[c][0]).view(F))
             nInt[r] = max(nInt.get(r, F(0.0)), m)
+            if variant == 2:
+                nsum[r] = nsum.get(r, 0) + csum[c]          # exact int64 sums
         size, Int = nsize, nInt
+        if variant == 2:
+            csum = nsum
         label = [rt[l] for l in label]
         medges = [(wb, idx, rt[a], rt[b]) for wb, idx, a, b in medges]
         levels += 1

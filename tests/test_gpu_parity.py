@@ -51,7 +51,9 @@ def test_synth_generator_matches_oracle(gseg, oracle, seg):
 @pytest.mark.parametrize("conn", [4, 8])
 def test_blur_and_weights_bit_exact(gseg, oracle, seg, w, h, conn):
     img = oracle.synth(w, h, 100 + w)
-    for sigma in (0.8, 0.0, 1.7, 2.6):  # 2.6: more than 8 one-sided taps -> the general (non-tile) blur kernels
+    # 0.25 R lands on k_blur_tile<R> (0.8 and 1.7 are R = 4 and 7); 2.0 is the last tile sigma, its float successor and
+    # 2.6 have more than 8 one-sided taps -> the general (non-tile) blur kernels
+    for sigma in (0.8, 0.0, 0.5, 0.75, 1.25, 1.5, 1.7, 2.0, float(np.nextafter(np.float32(2.0), np.float32(3.0))), 2.6):
         seg.segment(img, sigma=sigma, k=300, min_size=0, connectivity=conn, variant=gseg.FELZ)
         pl = oracle.blur(img, sigma)
         assert np.array_equal(seg.blurred().view(np.uint32), pl.view(np.uint32))
@@ -288,20 +290,20 @@ def test_adversarial_full_size_inputs(gseg, oracle, seg):
 
 
 def test_sort_pairs(gseg, seg):
+    """Sorted as unsigned 64-bit keys by their bits [begin, end), stably: numpy's stable argsort of that field."""
     import torch
-    for n, bits in [(1, 64), (1000, 64), (4096, 40), (100003, 64), (3_000_000, 52), (5_000_000, 64)]:
-        g = torch.Generator(device="cuda").manual_seed(n)
-        keys = torch.randint(0, 2 ** 62, (n,), dtype=torch.int64, device="cuda", generator=g)
-        if bits < 64:
-            keys &= (1 << bits) - 1
-        keys[::7] = int(keys[0].item())  # duplicates: stability must keep payload order
-        vals = torch.arange(n, dtype=torch.int32, device="cuda")
-        ref_k, ref_i = torch.sort(keys, stable=True)
-        k2, v2 = keys.clone(), vals.clone()
+    for n, begin, end in [(1, 0, 64), (1000, 0, 64), (4096, 0, 40), (100003, 0, 64), (3_000_000, 0, 52), (5_000_000, 0, 64),
+                          (4095, 0, 64), (4097, 8, 40), (8193, 13, 29), (100003, 60, 64), (1_000_003, 63, 64), (65536, 0, 1)]:
+        rng = np.random.default_rng(n + begin)
+        keys = rng.integers(0, 2 ** 64, n, dtype=np.uint64)   # every bit, the top two included
+        keys[::7] = keys[0]  # duplicates: stability must keep payload order
+        order = np.argsort((keys >> np.uint64(begin)) & np.uint64((1 << (end - begin)) - 1), kind="stable")
+        k2 = torch.from_numpy(keys.view(np.int64)).cuda()
+        v2 = torch.arange(n, dtype=torch.int32, device="cuda")
         torch.cuda.synchronize()  # the sort runs on the context's own stream: its inputs must be complete (torch wrote them on another)
-        seg.sort_pairs(k2.data_ptr(), v2.data_ptr(), n, 0, bits)
-        assert torch.equal(k2, ref_k)
-        assert torch.equal(v2.long(), ref_i)
+        seg.sort_pairs(k2.data_ptr(), v2.data_ptr(), n, begin, end)
+        assert np.array_equal(k2.cpu().numpy().view(np.uint64), keys[order]), (n, begin, end)
+        assert np.array_equal(v2.cpu().numpy(), order), (n, begin, end)
 
 
 def test_cli_ppm_roundtrip(gseg, oracle, tmp_path):

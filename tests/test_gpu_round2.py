@@ -195,10 +195,11 @@ def test_segment_graph_rejects_unordered_floats(gseg, seg):
 
 def test_strip_with_halo_equals_untiled_blur_and_weights(gseg, oracle, seg):
     """A strip segmented with its halo rows has the untiled image's blurred pixels and edge weights, bit for bit --
-    for the tile blur (sigma 0.8, 1.7) and the general blur (sigma 2.6: more than 8 taps)."""
+    for the tile blur (every template: sigma 0.25 R, R = 1..8; 0.8 and 1.7 are R = 4 and 7) and the general blur
+    (sigma 2.6: more than 8 taps)."""
     tiled = importlib.import_module(gseg.__name__ + ".tiled")
     img = oracle.synth(150, 200, 21)
-    for sigma in (0.8, 1.7, 2.6):
+    for sigma in (0.8, 1.7, 2.6, 0.25, 0.5, 0.75, 1.0, 1.25, 1.5, 1.75, 2.0):
         whole = oracle.blur(img, sigma)
         for i in range(3):
             y0, y1, ht, hb = tiled.strip_with_halo(200, 3, i, sigma)

@@ -155,6 +155,24 @@ def test_round_cap_and_level_cap(oracle):
     assert len(r2["stats"]) == 2
 
 
+@pytest.mark.parametrize("w,h,seed", [(12, 9, 1), (16, 16, 2), (9, 4, 5), (1, 6, 4)])
+@pytest.mark.parametrize("conn", [4, 8])
+def test_superpix_matches_pyref(oracle, w, h, seed, conn):
+    """The superpixel variant restated: Sobel, strength and every level (per-round mean-colour re-weighting with
+    24.8 fixed-point sums) against the oracle."""
+    img = oracle.synth(w, h, seed)
+    pl = oracle.blur(img, 0.8)
+    G = oracle.sobel(pl)
+    np.testing.assert_array_equal(G.view(np.uint32), pyref.sobel(pl).view(np.uint32))
+    es, sref = pyref.strength_list(G, conn)
+    np.testing.assert_array_equal(oracle.strength(G, conn).view(np.uint32), sref.view(np.uint32))
+    r = oracle.pipeline(img, 0.8, 0.0, 0, conn, oracle.SUPERPIX, max_levels=64)
+    _, levels = pyref.boruvka(es, w * h, 2, planes=pl)
+    assert r["nlevels"] == len(levels) and (r["n"] == 1 or w * h == 1)
+    for a, b in zip(r["levels"], levels):
+        assert np.array_equal(oracle.canon(a)[0].reshape(-1), pyref.canon(b))
+
+
 def test_superpix_runs_and_nests(oracle):
     w, h = 48, 36
     img = oracle.synth(w, h, 3)
