@@ -725,10 +725,19 @@ static void launch_r0_graph(gseg_ctx *c, cudaStream_t s, int ntiles, const GsegB
     if (!attr[c->device & 63]) { cudaFuncSetAttribute(k_r0_graph<VARIANT, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)graph_smem<VARIANT, D>()); attr[c->device & 63] = true; }
     k_r0_graph<VARIANT, D><<<ntiles < c->num_sms * c->occ_mult ? ntiles : c->num_sms * c->occ_mult, NT, graph_smem<VARIANT, D>(), s>>>(c->d_ctl, B);
 }
+// Staging the next page in shared memory pays while a warp has few pages: the pool's images (7 pages per warp at
+// 1080p, ~55 for 4K 8-connected) ran 3-4 % faster end to end; one 2^30-pixel image alone (~1 800 pages per warp)
+// ran 0.9 % slower, so beyond this many pages per warp the rows are loaded straight into registers.
+#define R0_STAGE_MAX_PPW 128
 template <int D, bool SP>
 static void launch_r0_edges(gseg_ctx *c, cudaStream_t s, size_t V, const GsegBufs &B) {
-    const size_t ntiles = ((size_t)D * ((V + GSEG_PAGE - 1) / GSEG_PAGE) + NT / 32 - 1) / (NT / 32); // blocks that cover all pages
-    k_r0_edges<D, SP><<<(int)(ntiles < (size_t)c->num_sms * c->occ_mult ? ntiles : (size_t)c->num_sms * c->occ_mult), NT, 0, s>>>(c->d_ctl, B);
+    static bool attr[64] = {false};
+    if (!attr[c->device & 63]) { cudaFuncSetAttribute(k_r0_edges<D, SP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)R0_SMEM); attr[c->device & 63] = true; }
+    const size_t pages = (size_t)D * ((V + GSEG_PAGE - 1) / GSEG_PAGE);
+    const size_t ntiles = (pages + NT / 32 - 1) / (NT / 32); // blocks that cover all pages
+    const int grid = (int)(ntiles < (size_t)c->num_sms * c->occ_mult ? ntiles : (size_t)c->num_sms * c->occ_mult);
+    if (pages <= (size_t)R0_STAGE_MAX_PPW * grid * (NT / 32)) k_r0_edges<D, SP, true><<<grid, NT, R0_SMEM, s>>>(c->d_ctl, B);
+    else k_r0_edges<D, SP, false><<<grid, NT, 0, s>>>(c->d_ctl, B);
 }
 
 // Round 0: blur -> [sobel] -> fused graph kernel -> relabel -> edge list.  4-5 launches.

@@ -708,6 +708,58 @@ __device__ __forceinline__ void emit_row_east(const GsegBufs &B, int nxt, u32 po
 #endif
 }
 
+// Per-warp bulk copies global -> shared (cp.async.bulk, completion counted in bytes on an mbarrier).
+__device__ __forceinline__ u32 smem_addr(const void *p) { return (u32)__cvta_generic_to_shared(p); }
+__device__ __forceinline__ void mbar_init(u64 *bar) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;\n\tfence.mbarrier_init.release.cluster;" ::"r"(smem_addr(bar)) : "memory");
+}
+__device__ __forceinline__ void mbar_expect_tx(u64 *bar, u32 bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_addr(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(u64 *bar, u32 parity) {
+    asm volatile("{\n\t.reg .pred P1;\n\tWAIT:\n\t"
+                 "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n\t"
+                 "@!P1 bra WAIT;\n\t}" ::"r"(smem_addr(bar)), "r"(parity) : "memory");
+}
+// src and dst 16-byte aligned, bytes a non-zero multiple of 16
+__device__ __forceinline__ void bulk_copy(void *dst, const void *src, u32 bytes, u64 *bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"(smem_addr(dst)), "l"(src), "r"(bytes), "r"(smem_addr(bar)) : "memory");
+}
+// shared memory the warp read with ordinary loads is about to be overwritten by a bulk copy
+__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+
+// Round-0 edge page staging.  A page of direction d reads three streams: map[p] (a ends), map[p + off] (b ends)
+// and the weights wgrid[d V + p], p in [p0, min(p0 + 256, V)); only the b stream can start below 0 (NE: off < 0)
+// or end past V, and it is clipped to [0, V) (a lane whose b end lies outside is masked anyway).  Each stream is
+// copied from the 16-byte boundary at or below its first word to the one at or above its last word: up to 3
+// words beyond the live range at each end, inside the allocations (map sits in the arena, which holds >= V + 64
+// words; wgrid holds D (V + 64)).
+#define R0_STREAM 264                                    // u32 per staged stream: 256 + 2 x 3 alignment words, rounded to 16 B
+#define R0_BUF (3 * R0_STREAM)                           // one page: a ends, b ends, weights
+#define R0_SMEM ((NT / 32) * (2 * R0_BUF * 4 + 16))      // bytes per block: two page buffers and two mbarriers per warp
+struct R0Page {
+    int d, off; // direction, pixel offset of the b end
+    u32 p0;     // first pixel of the page
+    u32 src[3]; // 16-byte aligned first word of each stream: map (a), map (b), wgrid
+    u32 n[3];   // words to copy (multiple of 4, may be 0)
+};
+__device__ __forceinline__ R0Page r0_page(u32 tile, u32 tpd, u32 V, int w) {
+    R0Page pg;
+    pg.d = (int)(tile / tpd);
+    pg.off = pg.d == 0 ? 1 : pg.d == 1 ? w : pg.d == 2 ? w + 1 : 1 - w;
+    pg.p0 = (tile - (u32)pg.d * tpd) * GSEG_PAGE;
+    const long long end = min((long long)pg.p0 + GSEG_PAGE, (long long)V);
+    const long long lo[3] = {pg.p0, max((long long)pg.p0 + pg.off, 0LL), (long long)pg.d * V + pg.p0};
+    const long long hi[3] = {end, min(end + pg.off, (long long)V), (long long)pg.d * V + end};
+#pragma unroll
+    for (int s = 0; s < 3; ++s) {
+        pg.src[s] = (u32)(lo[s] & ~3LL);
+        pg.n[s] = hi[s] > lo[s] ? (u32)(((hi[s] + 3) & ~3LL) - (lo[s] & ~3LL)) : 0u;
+    }
+    return pg;
+}
+
 // a10 (round 0): grid edges -> paged list of inter-component edges, in edge-index order
 // (direction-major: all E edges in pixel order, then S, SE, NE).
 //
@@ -721,37 +773,108 @@ __device__ __forceinline__ void emit_row_east(const GsegBufs &B, int nxt, u32 po
 // together, each look-back walks back through thousands of not-yet-resolved predecessors.)  Only when
 // the pages have become sparse (< 1/4 full) does one round re-pack the list densely with the ordered
 // scan; by then the list is small.
-template <int D, bool SP>
+//
+// STAGED: every page starts with three dependent-free 1 KB reads whose addresses are known long before:
+// each warp keeps two page buffers in shared memory and bulk-copies page t + nw into one while it works
+// on page t from the other, so the reads of a page overlap the emits of the one before.  Otherwise the
+// page's rows are loaded straight into registers (the host picks by pages per warp, R0_STAGE_MAX_PPW).
+template <int D, bool SP, bool STAGED>
 __global__ void __launch_bounds__(NT, GSEG_LB_EDGES) k_r0_edges(GsegCtl *ctl, GsegBufs B) {
     constexpr int ROWS = GSEG_PAGE / 32;
-    const int lane = threadIdx.x & 31;
+    extern __shared__ __align__(16) u32 r0_stage[]; // R0_SMEM bytes: [NT / 32][2] mbarriers, then [NT / 32][2][R0_BUF]
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const u32 lt = (1u << lane) - 1u;
     const RoundState st = ctl->st; // round 0
     const int w = ctl->p.w, h = ctl->p.h;
     const u32 V = (u32)w * (u32)h;
     const u32 *__restrict__ map = B.arena; // round 0's map sits at arena offset 0
+    const u32 *__restrict__ wgrid = reinterpret_cast<const u32 *>(B.wgrid);
     const u32 tpd = (V + GSEG_PAGE - 1) / GSEG_PAGE, ntiles = tpd * (u32)D;
     const u32 nw = gridDim.x * (NT / 32);
+    u64 *bar = reinterpret_cast<u64 *>(r0_stage) + 2 * wid;
+    u32 *buf = r0_stage + 4 * (NT / 32) + wid * 2 * R0_BUF;
+    auto stage = [&](u32 tile, u32 k) { // lane 0: start the copies of page `tile` into buffer k
+        const R0Page pg = r0_page(tile, tpd, V, w);
+        u32 *dst = buf + k * R0_BUF;
+        fence_proxy_async();
+        mbar_expect_tx(bar + k, 4u * (pg.n[0] + pg.n[1] + pg.n[2]));
+        bulk_copy(dst, map + pg.src[0], 4u * pg.n[0], bar + k); // the a stream is never empty
+        if (pg.n[1]) bulk_copy(dst + R0_STREAM, map + pg.src[1], 4u * pg.n[1], bar + k);
+        bulk_copy(dst + 2 * R0_STREAM, wgrid + pg.src[2], 4u * pg.n[2], bar + k);
+    };
     u32 esum = 0;
     if (blockIdx.x == 0 && threadIdx.x == 0) ctl->ticketC = 0;
-    for (u32 tile = blockIdx.x * (NT / 32) + (threadIdx.x >> 5); tile < ntiles; tile += nw) {
-        const int d = (int)(tile / tpd);
+    u32 tile = blockIdx.x * (NT / 32) + wid;
+    if constexpr (!STAGED) {
+        for (; tile < ntiles; tile += nw) {
+            const int d = (int)(tile / tpd);
+            const int dx = d == 1 ? 0 : 1, dy = d == 0 ? 0 : (d == 3 ? -1 : 1);
+            const int off = dy * w + dx;
+            const u32 p0 = (tile - (u32)d * tpd) * GSEG_PAGE + lane;
+            u32 a[ROWS], b[ROWS], m[ROWS], wv[ROWS];
+            const u32 *wg = wgrid + (size_t)d * V + p0;
+            int y = (int)(p0 / (u32)w), x = (int)(p0 - (u32)y * (u32)w);
+#pragma unroll
+            for (int j = 0; j < ROWS; ++j) {
+                const u32 p = p0 + 32u * j;
+                bool keep = false;
+                a[j] = b[j] = wv[j] = 0u;
+                if (p < V && x + dx < w && y + dy < h && y + dy >= 0) {
+                    a[j] = map[p];
+                    b[j] = map[(u32)((int)p + off)];
+                    wv[j] = wg[32 * j]; // with the ids, not row by row between the emits: one round trip per page
+                    keep = a[j] != b[j];
+                }
+                m[j] = __ballot_sync(0xFFFFFFFFu, keep);
+                x += 32;
+                while (x >= w) { x -= w; ++y; }
+            }
+            u32 total = 0;
+#pragma unroll
+            for (int j = 0; j < ROWS; ++j) total += __popc(m[j]);
+            if (lane == 0) { B.pcnt[1][tile] = total; B.poff[1][tile] = tile * GSEG_PAGE; }
+            GSEG_CHK(ctl, (unsigned long long)tile * GSEG_PAGE + total <= ctl->p.edge_slots, 4);
+            esum += total;
+            u32 rowoff = tile * GSEG_PAGE;
+#pragma unroll
+            for (int j = 0; j < ROWS; ++j) {
+                if (m[j] == 0u) continue; // warp-uniform
+                const bool act = (m[j] >> lane) & 1u;
+                if (d == 0) emit_row_east<SP>(B, 1, rowoff + __popc(m[j] & lt), act, a[j], b[j], wv[j]);
+                else emit_row<SP, false>(B, 1, rowoff + __popc(m[j] & lt), act, a[j], b[j], wv[j]);
+                rowoff += __popc(m[j]);
+            }
+        }
+    } else {
+    if (lane == 0) {
+        mbar_init(bar);
+        mbar_init(bar + 1);
+        if (tile < ntiles) stage(tile, 0u);
+    }
+    __syncwarp();
+    for (u32 it = 0; tile < ntiles; tile += nw, ++it) {
+        const u32 k = it & 1u;
+        __syncwarp(); // every lane has finished reading buffer k ^ 1 (page tile - nw): refill it
+        if (lane == 0 && tile + nw < ntiles) stage(tile + nw, k ^ 1u);
+        const R0Page pg = r0_page(tile, tpd, V, w);
+        const int d = pg.d, off = pg.off;
         const int dx = d == 1 ? 0 : 1, dy = d == 0 ? 0 : (d == 3 ? -1 : 1);
-        const int off = dy * w + dx;
-        const u32 p0 = (tile - (u32)d * tpd) * GSEG_PAGE + lane;
-        u32 a[ROWS], b[ROWS], m[ROWS], wv[ROWS];
-        const float *wg = B.wgrid + (size_t)d * V + p0;
+        const u32 p0 = pg.p0 + lane;
+        const u32 *sa = buf + k * R0_BUF + lane;                                          // map[p0 + i]
+        const u32 *sb = buf + k * R0_BUF + R0_STREAM + (int)(pg.p0 + off - pg.src[1]) + lane; // map[p0 + off + i]
+        const u32 *sw = buf + k * R0_BUF + 2 * R0_STREAM + (d * V + pg.p0 - pg.src[2]) + lane; // wgrid[d V + p0 + i]
+        // rows are read from the buffer twice (for the survivor ballots, then for the emits) instead of being
+        // held in registers across the emits: 8 rows x (a, b, w) registers less, no spills
+        u32 m[ROWS], live = 0u; // live bit j: row j's edge exists (inside the image)
         int y = (int)(p0 / (u32)w), x = (int)(p0 - (u32)y * (u32)w);
+        mbar_wait(bar + k, (it >> 1) & 1u);
 #pragma unroll
         for (int j = 0; j < ROWS; ++j) {
             const u32 p = p0 + 32u * j;
             bool keep = false;
-            a[j] = b[j] = wv[j] = 0u;
             if (p < V && x + dx < w && y + dy < h && y + dy >= 0) {
-                a[j] = map[p];
-                b[j] = map[(u32)((int)p + off)];
-                wv[j] = __float_as_uint(wg[32 * j]); // with the ids, not row by row between the emits: one round trip per page
-                keep = a[j] != b[j];
+                live |= 1u << j;
+                keep = sa[32 * j] != sb[32 * j];
             }
             m[j] = __ballot_sync(0xFFFFFFFFu, keep);
             x += 32;
@@ -767,11 +890,13 @@ __global__ void __launch_bounds__(NT, GSEG_LB_EDGES) k_r0_edges(GsegCtl *ctl, Gs
 #pragma unroll
         for (int j = 0; j < ROWS; ++j) {
             if (m[j] == 0u) continue; // warp-uniform
-            const bool act = (m[j] >> lane) & 1u;
-            if (d == 0) emit_row_east<SP>(B, 1, rowoff + __popc(m[j] & lt), act, a[j], b[j], wv[j]);
-            else emit_row<SP, false>(B, 1, rowoff + __popc(m[j] & lt), act, a[j], b[j], wv[j]);
+            const bool act = (m[j] >> lane) & 1u, in = (live >> j) & 1u;
+            const u32 a = in ? sa[32 * j] : 0u, b = in ? sb[32 * j] : 0u, wv = in ? sw[32 * j] : 0u;
+            if (d == 0) emit_row_east<SP>(B, 1, rowoff + __popc(m[j] & lt), act, a, b, wv);
+            else emit_row<SP, false>(B, 1, rowoff + __popc(m[j] & lt), act, a, b, wv);
             rowoff += __popc(m[j]);
         }
+    }
     }
     if (lane == 0 && esum) atomicAdd(&ctl->Eacc[0], esum);
     RoundState s0 = st;
