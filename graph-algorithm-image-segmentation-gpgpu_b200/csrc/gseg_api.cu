@@ -38,6 +38,11 @@ static_assert(offsetof(GsegCtl, resume_phase) == offsetof(GsegHead, resume_phase
 static_assert(offsetof(GsegCtl, stDedupOut) == offsetof(GsegHead, stDedupOut), "GsegHead must mirror the head of GsegCtl");
 #define GSEG_EPOCHS_PER_RUN (2u * GSEG_MAXR + 8u + 32u) /* look-back tags a run may use: 2 per round, 8 spare, 32 de-duplications */
 
+// Staging the next page in shared memory pays while a warp has few pages: the pool's images (7 pages per warp at
+// 1080p, ~55 for 4K 8-connected) ran 3-4 % faster end to end; one 2^30-pixel image alone (~1 800 pages per warp)
+// ran 0.9 % slower, so beyond this many pages per warp the rows are loaded straight into registers.
+#define R0_STAGE_MAX_PPW 128
+
 static const size_t TAIL_SMEM = (2 * (size_t)GSEG_TAIL_STAGE + 2 * (NTT / 32)) * sizeof(u32); // k_tail: staged map + minima, survivor-count exchange (phase_E)
 
 struct gseg_ctx {
@@ -63,6 +68,7 @@ struct gseg_ctx {
     GsegHead *h_head; // pinned image of the host-initialised head of the control block
     int num_sms, occ_mult;
     u32 filter_shift;
+    u32 r0_stage_ppw;     // round-0 edge kernel: most pages per warp for the staged body (GSEG_R0_STAGE_PPW)
     int tail_cluster;     // CTAs in the tail kernel's cluster (16 non-portable, else 8)
     bool tail_cluster_env; // GSEG_TAIL_CLUSTER was given: a pool leaves the size alone
     u32 tail_E, tail_V, tail_P; // hand-over thresholds of the tail kernel
@@ -297,6 +303,8 @@ extern "C" int gseg_create_ex(gseg_ctx **out, int device, int max_w, int max_h, 
         if (const char *ev = getenv("GSEG_OCC_MULT")) ctx->occ_mult = atoi(ev) > 0 ? atoi(ev) : 4;
         ctx->filter_shift = 6;
         if (const char *ev = getenv("GSEG_FILTER_SHIFT")) ctx->filter_shift = (u32)atoi(ev);
+        ctx->r0_stage_ppw = R0_STAGE_MAX_PPW; // test knob: 0 = always the register body, huge = always the staged one
+        if (const char *ev = getenv("GSEG_R0_STAGE_PPW")) ctx->r0_stage_ppw = (u32)strtoul(ev, nullptr, 10);
     }
     if (e != cudaSuccess) {
         fprintf(stderr, "gseg_create: %s\n", cudaGetErrorString(e));
@@ -725,10 +733,6 @@ static void launch_r0_graph(gseg_ctx *c, cudaStream_t s, int ntiles, const GsegB
     if (!attr[c->device & 63]) { cudaFuncSetAttribute(k_r0_graph<VARIANT, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)graph_smem<VARIANT, D>()); attr[c->device & 63] = true; }
     k_r0_graph<VARIANT, D><<<ntiles < c->num_sms * c->occ_mult ? ntiles : c->num_sms * c->occ_mult, NT, graph_smem<VARIANT, D>(), s>>>(c->d_ctl, B);
 }
-// Staging the next page in shared memory pays while a warp has few pages: the pool's images (7 pages per warp at
-// 1080p, ~55 for 4K 8-connected) ran 3-4 % faster end to end; one 2^30-pixel image alone (~1 800 pages per warp)
-// ran 0.9 % slower, so beyond this many pages per warp the rows are loaded straight into registers.
-#define R0_STAGE_MAX_PPW 128
 template <int D, bool SP>
 static void launch_r0_edges(gseg_ctx *c, cudaStream_t s, size_t V, const GsegBufs &B) {
     static bool attr[64] = {false};
@@ -736,8 +740,14 @@ static void launch_r0_edges(gseg_ctx *c, cudaStream_t s, size_t V, const GsegBuf
     const size_t pages = (size_t)D * ((V + GSEG_PAGE - 1) / GSEG_PAGE);
     const size_t ntiles = (pages + NT / 32 - 1) / (NT / 32); // blocks that cover all pages
     const int grid = (int)(ntiles < (size_t)c->num_sms * c->occ_mult ? ntiles : (size_t)c->num_sms * c->occ_mult);
-    if (pages <= (size_t)R0_STAGE_MAX_PPW * grid * (NT / 32)) k_r0_edges<D, SP, true><<<grid, NT, R0_SMEM, s>>>(c->d_ctl, B);
-    else k_r0_edges<D, SP, false><<<grid, NT, 0, s>>>(c->d_ctl, B);
+    // profiled as k_r0_edges (staged body) or k_r0_edges_rl (register-load body)
+    if (pages <= (size_t)c->r0_stage_ppw * grid * (NT / 32)) {
+        mark(c, s, "k_r0_edges", 0);
+        k_r0_edges<D, SP, true><<<grid, NT, R0_SMEM, s>>>(c->d_ctl, B);
+    } else {
+        mark(c, s, "k_r0_edges_rl", 0);
+        k_r0_edges<D, SP, false><<<grid, NT, 0, s>>>(c->d_ctl, B);
+    }
 }
 
 // Round 0: blur -> [sobel] -> fused graph kernel -> relabel -> edge list.  4-5 launches.
@@ -782,7 +792,6 @@ static void enqueue_round0(gseg_ctx *c, cudaStream_t s) {
         mark(c, s, "k_means", 0);
         k_means<<<grid_for(V, NT, c->num_sms * c->occ_mult), NT, 0, s>>>(c->d_ctl, B);
     }
-    mark(c, s, "k_r0_edges", 0);
     if (D == 2) { if (sp) launch_r0_edges<2, true>(c, s, V, B); else launch_r0_edges<2, false>(c, s, V, B); }
     else { if (sp) launch_r0_edges<4, true>(c, s, V, B); else launch_r0_edges<4, false>(c, s, V, B); }
 }
@@ -1812,7 +1821,7 @@ static void algo_bytes(const gseg_ctx *c, const char *name, int r, double *algo,
         s = 4 * V + 4 * Vn + 4 * V + attr_in + 4 * (V - Vn) + out; // the chain is inside succ[], the ids gathered are Vn distinct words
     }
     // grid edges: weight in (the ends are implicit), both ends' new ids gathered (4 + 4), survivors out (12), one minimum per component
-    else if (!strcmp(name, "k_r0_edges")) { a = 4 * E0 + 8 * E0 + 12 * En + 8 * Vn; s = 4 * E0 + 4 * V0 + 12 * En + 8 * Vn; }
+    else if (!strcmp(name, "k_r0_edges") || !strcmp(name, "k_r0_edges_rl")) { a = 4 * E0 + 8 * E0 + 12 * En + 8 * Vn; s = 4 * E0 + 4 * V0 + 12 * En + 8 * Vn; }
     // per component: its minimum in (8), that edge's ends gathered (8), (size, Int) of both ends (16) and the partner's
     // minimum (8) gathered; successor + chosen weight out (8); new id of every root + its cleared accumulators
     else if (!strcmp(name, "k_succ_scan")) { a = 8 * V + 8 * V + 16 * V + 8 * V + 8 * V + (4 + acc) * Vn; s = 8 * V + 8 * V + 8 * V + 8 * V + (4 + acc) * Vn; }

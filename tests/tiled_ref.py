@@ -22,6 +22,23 @@ def dedup_edges(ea, eb, w):
     return ea[keep].astype(np.uint32), eb[keep].astype(np.uint32), w[keep]
 
 
+def grid_edges(labels, wts, w, h, conn):
+    """(ea, eb, w) of the grid edges whose ends carry different labels, in edge-index order (direction-major: E, S, SE,
+    NE, then pixel order), ends mapped through the label image and weights taken from wts[d * V + p]."""
+    lab = np.asarray(labels).reshape(-1)
+    V = h * w
+    ys, xs = np.divmod(np.arange(V), w)
+    dirs = [(1, 0), (0, 1)] + ([(1, 1), (1, -1)] if conn == 8 else [])
+    ea, eb, ww = [], [], []
+    for d, (dx, dy) in enumerate(dirs):
+        ok = (xs + dx < w) & (ys + dy < h) & (ys + dy >= 0)
+        p = np.nonzero(ok)[0]
+        q = p + dy * w + dx
+        keep = lab[p] != lab[q]
+        ea.append(lab[p[keep]]); eb.append(lab[q[keep]]); ww.append(wts[d * V + p[keep]])
+    return np.concatenate(ea), np.concatenate(eb), np.concatenate(ww).astype(np.float32)
+
+
 def oracle_strip(O, img, sigma, k, min_size, conn, max_rounds=48, dedup=True, halo_top=0, halo_bottom=0):
     """(dense labels, graph, top colours, bottom colours) of one strip, from the CPU oracle.  img holds halo_top rows
     above and halo_bottom rows below the strip: they take part in the blur only."""
@@ -38,18 +55,7 @@ def oracle_strip(O, img, sigma, k, min_size, conn, max_rounds=48, dedup=True, ha
     first[dense[::-1]] = rep[::-1]
     size = np.bincount(dense, minlength=n).astype(np.uint32)
     Int = r["int"][first]
-    # live edges in edge-index order: direction-major, then pixel order
-    V = h * w
-    ys, xs = np.divmod(np.arange(V), w)
-    dirs = [(1, 0), (0, 1)] + ([(1, 1), (1, -1)] if conn == 8 else [])
-    ea, eb, ww = [], [], []
-    for d, (dx, dy) in enumerate(dirs):
-        ok = (xs + dx < w) & (ys + dy < h) & (ys + dy >= 0)
-        p = np.nonzero(ok)[0]
-        q = p + dy * w + dx
-        keep = dense[p] != dense[q]
-        ea.append(dense[p[keep]]); eb.append(dense[q[keep]]); ww.append(wts[d * V + p[keep]])
-    ea, eb, ww = np.concatenate(ea), np.concatenate(eb), np.concatenate(ww).astype(np.float32)
+    ea, eb, ww = grid_edges(dense, wts, w, h, conn)
     if dedup:
         ea, eb, ww = dedup_edges(ea, eb, ww)
     graph = dict(size=size, Int=Int.astype(np.float32), ea=ea.astype(np.uint32), eb=eb.astype(np.uint32), w=ww)

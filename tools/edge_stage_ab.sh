@@ -24,7 +24,7 @@ for sz in "1920 1080" "16384 8192"; do
   for t in OLD NEW; do
     tag=$(echo $sz | tr ' ' x)_c4_v0
     (cd "${!t}" && GSEG_NOBUILD=1 python tools/prof.py $sz 4 0 > "$OUT/prof_${tag}_$t.txt" 2>&1)
-    echo "== prof $sz $t"; grep -E "^k_r0_edges +0|^k_edges +[1-4] |persistent" "$OUT/prof_${tag}_$t.txt"
+    echo "== prof $sz $t"; grep -E "^k_r0_edges(_rl)? +0|^k_edges +[1-4] |persistent" "$OUT/prof_${tag}_$t.txt"
   done
 done
 DUMP=$(mktemp -d)
