@@ -25,9 +25,10 @@ FELZ, HIER, SUPERPIX = 0, 1, 2
 MEM_HOST, MEM_DEVICE = 0, 1
 FLAG_HOST_LOOP = 1
 FLAG_NO_DEDUP = 2
-CAP_SUPERPIX, CAP_WIDE_SIGMA, CAP_LEVELS, CAP_JPEG = 1, 2, 4, 8
+CAP_SUPERPIX, CAP_WIDE_SIGMA, CAP_LEVELS, CAP_JPEG, CAP_REGIONS = 1, 2, 4, 8, 16
 JPEG_AUTO, JPEG_OWN, JPEG_NVJPEG = 0, 1, 2  # decoders behind gseg_segment_jpeg (include/gseg.h)
-OUT_NONE, OUT_LABELS, OUT_HIERARCHY = 0, 1, 2
+OUT_NONE, OUT_LABELS, OUT_HIERARCHY, OUT_REGIONS = 0, 1, 2, 3
+RENDER_MEAN, RENDER_OVERLAY, RENDER_BOUNDARY = 0, 1, 2  # gseg_render modes
 POOL_MAXLEVELS = 64
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
@@ -135,6 +136,9 @@ def load():
     L.gseg_sync.argtypes = [vp]
     L.gseg_labels_all.argtypes = [vp, vp, i32, i32]
     L.gseg_colorize.argtypes = [vp, i32, u64, vp, i32]
+    L.gseg_regions.argtypes = [vp, i32, vp, i32, i32, vp, C.c_int64, i32]
+    L.gseg_regions_async.argtypes = [vp, i32, vp, i32, i32, vp, C.c_int64, i32]
+    L.gseg_render.argtypes = [vp, i32, i32, C.c_uint32, vp, i32, i32, vp, i32]
     L.gseg_weights.argtypes = [vp, vp, i32]
     L.gseg_blurred.argtypes = [vp, vp, i32]
     L.gseg_stats.argtypes = [vp, C.POINTER(RoundStat), i32]
@@ -224,6 +228,19 @@ def jpeg_info(data):
     if rc:
         raise GsegError("gseg_jpeg_info: %s" % L.gseg_strerror(rc).decode())
     return int(w.value), int(h.value)
+
+
+def regions_frame(table):
+    """Named columns of a region table ((n, 8) uint64 from Segmenter.regions): count, mean colour (rounded as
+    gseg_render's mean picture: (sum + count // 2) // count), centroid (float64) and inclusive bounding box."""
+    t = np.asarray(table, np.uint64).reshape(-1, 8)
+    n = np.maximum(t[:, 0], 1)
+    mean = (t[:, 1:4] + (n // 2)[:, None]) // n[:, None]
+    lo32 = np.uint64(0xFFFFFFFF)
+    return dict(count=t[:, 0].astype(np.int64), mean_rgb=mean.astype(np.uint8),
+                centroid_x=t[:, 4] / n.astype(np.float64), centroid_y=t[:, 5] / n.astype(np.float64),
+                x0=(t[:, 6] & lo32).astype(np.int64), y0=(t[:, 6] >> np.uint64(32)).astype(np.int64),
+                x1=(t[:, 7] & lo32).astype(np.int64), y1=(t[:, 7] >> np.uint64(32)).astype(np.int64))
 
 
 def _is_torch(x):
@@ -435,6 +452,42 @@ class Segmenter:
             out = np.empty((self.hh, self.w, 3), np.uint8)
         ptr, kind = _ptr(out)
         self._ck(self.L.gseg_colorize(self.h, level, seed, C.c_void_p(ptr), kind), "gseg_colorize")
+        return out
+
+    def _input_arg(self, rgb):
+        if rgb is None:
+            return None, 0, MEM_HOST
+        if _is_torch(rgb):
+            stride = int(rgb.stride(0)) * int(rgb.element_size())
+        else:
+            stride = int(rgb.strides[0])
+        ptr, kind = _ptr(rgb)
+        return C.c_void_p(ptr), stride, kind
+
+    def regions(self, level=-1, rgb=None, out=None, wait=True):
+        """Per-component statistics of a level as an (n, 8) uint64 array (gseg_regions; columns: count, sum r, g, b,
+        sum x, sum y, x0 | y0 << 32, x1 | y1 << 32; see regions_frame).  rgb: the image the run read, needed when it
+        was caller-owned device memory (None: the context's staged input).  out: a CUDA tensor keeps the table on the
+        device; wait=False only enqueues it (out must then be a CUDA tensor or pinned host memory)."""
+        n = self.num_components(level)
+        if out is None:
+            out = np.empty((n, 8), np.uint64)
+        cap = (int(out.numel() * out.element_size()) if _is_torch(out) else int(out.nbytes)) // 64
+        ptr, kind = _ptr(out)
+        rp, stride, rkind = self._input_arg(rgb)
+        fn = self.L.gseg_regions if wait else self.L.gseg_regions_async
+        self._ck(fn(self.h, level, rp, stride, rkind, C.c_void_p(ptr), cap, kind), "gseg_regions")
+        return out
+
+    def render(self, level=-1, mode=RENDER_MEAN, colour=0xFF0000, rgb=None, out=None):
+        """Picture of a level (gseg_render): RENDER_MEAN (each region's rounded mean colour), RENDER_OVERLAY (the input
+        with boundary pixels set to colour 0xRRGGBB) -> (h, w, 3) uint8; RENDER_BOUNDARY -> (h, w) uint8 mask.
+        out: numpy array or torch tensor (CUDA: the picture stays on the device)."""
+        if out is None:
+            out = np.empty((self.hh, self.w) if mode == RENDER_BOUNDARY else (self.hh, self.w, 3), np.uint8)
+        ptr, kind = _ptr(out)
+        rp, stride, rkind = self._input_arg(rgb)
+        self._ck(self.L.gseg_render(self.h, level, mode, colour, rp, stride, rkind, C.c_void_p(ptr), kind), "gseg_render")
         return out
 
     def weights(self):

@@ -108,10 +108,34 @@ class Pool:
                                                        self.L.gseg_pool_last_error(self.h).decode()))
         return rc
 
+    @staticmethod
+    def regions_out_bytes(w, h, max_components, elem_bytes=4):
+        """Bytes an OUT_REGIONS job writes at most: the label image, padding to 64 bytes, 64 bytes per component."""
+        return ((w * h * elem_bytes + 63) // 64) * 64 + 64 * max_components
+
+    @staticmethod
+    def split_regions(out, result):
+        """(label bytes, (n, 8) uint64 table) of an OUT_REGIONS job's host output `out` (numpy) and its result."""
+        raw = np.asarray(out).reshape(-1).view(np.uint8)
+        o1, o2 = int(result.offsets[1]), int(result.offsets[2])
+        return raw[:result.w * result.h * result.elem_bytes], raw[o1:o2].view(np.uint64).reshape(-1, 8)
+
     def jobs(self, images, outs, out_mode=1, level=-1, elem_bytes=0, **params):
         """A ctypes array of gseg_pool_job: images[i] (arrays / tensors of (h, w, 3) uint8, or bytes of a JPEG file)
-        -> outs[i] (array / tensor receiving the label image or the hierarchy; None with out_mode 0)."""
+        -> outs[i] (array / tensor receiving the label image, the hierarchy, or with OUT_REGIONS the label image and
+        the region table -- size it with regions_out_bytes; None with out_mode 0)."""
         g = self.gseg
+        if outs is None and out_mode == g.OUT_REGIONS:  # host buffers sized for the worst case (every pixel a component)
+            outs = []
+            for img in images:
+                if isinstance(img, Jpeg):
+                    buf = img.buf.numpy() if g._is_torch(img.buf) else np.asarray(img.buf)
+                    w, h = g.jpeg_info(buf.reshape(-1)[:img.nbytes].tobytes())
+                elif isinstance(img, (bytes, bytearray, memoryview)):
+                    w, h = g.jpeg_info(bytes(img))
+                else:
+                    h, w = int(img.shape[0]), int(img.shape[1])
+                outs.append(np.zeros(self.regions_out_bytes(w, h, w * h, elem_bytes or 4), np.uint8))
         arr = (g.PoolJob * len(images))()
         keep = []
         p = g.Params(params.get("sigma", 0.8), params.get("k", 300.0), params.get("min_size", 20), params.get("connectivity", 4),

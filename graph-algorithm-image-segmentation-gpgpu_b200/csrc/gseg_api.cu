@@ -17,6 +17,7 @@
 
 #include "../../include/gseg.h"
 #include "gseg_kernels.cuh"
+#include "gseg_regions.cuh"
 #include "gseg_sort.cuh"
 #include "gseg_dedup.cuh"
 #include "gseg_jpeg.hpp"
@@ -42,6 +43,12 @@ static_assert(offsetof(GsegCtl, stDedupOut) == offsetof(GsegHead, stDedupOut), "
 // 1080p, ~55 for 4K 8-connected) ran 3-4 % faster end to end; one 2^30-pixel image alone (~1 800 pages per warp)
 // ran 0.9 % slower, so beyond this many pages per warp the rows are loaded straight into registers.
 #define R0_STAGE_MAX_PPW 128
+
+// Region statistics: partitions with at most this many components accumulate in a block-private shared-memory table
+// (40 bytes per component: 40 KB at 1024, which leaves 5 blocks of 256 threads per SM); above it every warp's combined
+// runs go straight to 64-bit global atomics.  At 1024 components a block still sees only the few dozen regions its rows
+// cross, so the flush (one pass over the table, atomics for the non-empty records) stays small against its pixels.
+#define REGIONS_SMEM_MAX 1024
 
 static const size_t TAIL_SMEM = (2 * (size_t)GSEG_TAIL_STAGE + 2 * (NTT / 32)) * sizeof(u32); // k_tail: staged map + minima, survivor-count exchange (phase_E)
 
@@ -69,6 +76,10 @@ struct gseg_ctx {
     int num_sms, occ_mult;
     u32 filter_shift;
     u32 r0_stage_ppw;     // round-0 edge kernel: most pages per warp for the staged body (GSEG_R0_STAGE_PPW)
+    u32 rg_smem_max;      // region statistics: most components of the shared-memory tier (GSEG_REGIONS_SMEM_MAX)
+    u32 rg_smem_fit;      // ... and most the device's shared memory per block holds
+    u32 rg_n;             // components of the last region table (profile byte model)
+    u64 *d_rtab;          // region table staging for host output when d_best[0] is too small (GSEG_CAP_REGIONS)
     int tail_cluster;     // CTAs in the tail kernel's cluster (16 non-portable, else 8)
     bool tail_cluster_env; // GSEG_TAIL_CLUSTER was given: a pool leaves the size alone
     u32 tail_E, tail_V, tail_P; // hand-over thresholds of the tail kernel
@@ -305,6 +316,12 @@ extern "C" int gseg_create_ex(gseg_ctx **out, int device, int max_w, int max_h, 
         if (const char *ev = getenv("GSEG_FILTER_SHIFT")) ctx->filter_shift = (u32)atoi(ev);
         ctx->r0_stage_ppw = R0_STAGE_MAX_PPW; // test knob: 0 = always the register body, huge = always the staged one
         if (const char *ev = getenv("GSEG_R0_STAGE_PPW")) ctx->r0_stage_ppw = (u32)strtoul(ev, nullptr, 10);
+        ctx->rg_smem_max = REGIONS_SMEM_MAX; // test knob: 0 = always the global-atomic tier, huge = shared memory whenever it fits
+        if (const char *ev = getenv("GSEG_REGIONS_SMEM_MAX")) ctx->rg_smem_max = (u32)strtoul(ev, nullptr, 10);
+        int optin = 0;
+        e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, device);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(k_regions<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, optin);
+        ctx->rg_smem_fit = (u32)optin / (RG_FIELDS * sizeof(u32));
     }
     if (e != cudaSuccess) {
         fprintf(stderr, "gseg_create: %s\n", cudaGetErrorString(e));
@@ -608,7 +625,7 @@ extern "C" void gseg_destroy(gseg_ctx *ctx) {
     delete ctx->jplan;
     sort_scratch_free(&ctx->sort);
     cudaFree(ctx->d_xkeys); cudaFree(ctx->d_xvals); cudaFree(ctx->d_xkeep); cudaFree(ctx->d_xab); cudaFree(ctx->d_xw);
-    cudaFree(ctx->d_winner); cudaFree(ctx->d_dd);
+    cudaFree(ctx->d_winner); cudaFree(ctx->d_dd); cudaFree(ctx->d_rtab);
     for (int i = 0; i <= GSEG_MAXMARK; ++i)
         if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     if (ctx->h_ctl) cudaFreeHost(ctx->h_ctl);
@@ -999,7 +1016,7 @@ static int ensure_csum(gseg_ctx *ctx) {
 }
 
 extern "C" int gseg_reserve(gseg_ctx *ctx, uint32_t caps) {
-    if (!ctx || (caps & ~(GSEG_CAP_SUPERPIX | GSEG_CAP_WIDE_SIGMA | GSEG_CAP_LEVELS | GSEG_CAP_JPEG))) return GSEG_E_ARG;
+    if (!ctx || (caps & ~(GSEG_CAP_SUPERPIX | GSEG_CAP_WIDE_SIGMA | GSEG_CAP_LEVELS | GSEG_CAP_JPEG | GSEG_CAP_REGIONS))) return GSEG_E_ARG;
     if (ctx->pending) return GSEG_E_STATE;
     CK(cudaSetDevice(ctx->device));
     int rc = GSEG_OK;
@@ -1007,6 +1024,10 @@ extern "C" int gseg_reserve(gseg_ctx *ctx, uint32_t caps) {
     if (!rc && (caps & GSEG_CAP_WIDE_SIGMA)) rc = ensure(ctx, &ctx->d_tmp, 3 * (ctx->Vmax + 64));
     if (!rc && (caps & GSEG_CAP_LEVELS)) rc = ensure(ctx, &ctx->d_labels[1], ctx->Vmax + 64);
     if (!rc && (caps & GSEG_CAP_JPEG)) rc = jpeg_reserve_own(ctx, 0, 0, 0);
+    if (!rc && (caps & GSEG_CAP_REGIONS)) {
+        rc = ensure(ctx, &ctx->d_labels[1], ctx->Vmax + 64);
+        if (!rc) rc = ensure(ctx, &ctx->d_rtab, 8 * (ctx->Vmax + 64));
+    }
     return rc;
 }
 
@@ -1246,22 +1267,31 @@ static int level_to_round(const gseg_ctx *ctx, int level, int *round) {
 
 // Label image of the partition after round `round` into dst (device).  Deep hierarchies go through a
 // composed table of the late (small) rounds so that a pixel chases 3-4 maps instead of one per round.
-template <typename OutT>
-static void enqueue_compose(gseg_ctx *ctx, int round, OutT *dst) {
-    const size_t V = (size_t)ctx->w * ctx->h;
+// compose_table enqueues the table when the level is deep enough and returns it (else nullptr); a pixel then chases
+// the maps of rounds 1..*last and, with a table, looks its label up in it.  k_regions fuses the same chase.
+static const u32 *compose_table(gseg_ctx *ctx, int round, int *last) {
     const GsegCtl *h = ctx->h_ctl;
     int first = 1;
     while (first <= round && (h->stV[first] > 65536u || h->map_skip[first])) ++first; // first live round whose input has few components
     if (first >= 1 && first <= round && round - first >= 2 && h->stV[first] <= ctx->Vmax) {
         const u32 n = h->stV[first];
         u32 *F = ctx->d_wsel; // per-round scratch, free once the run is complete
-        ctx->launches += 2;
-        k_compose_table<<<grid_for(n, NT), NT, 0, ctx->stream>>>(ctx->d_ctl, ctx->d_arena, first, round, n, F);
-        k_compose_px<OutT><<<grid_for(V, NT), NT, 0, ctx->stream>>>(ctx->d_ctl, ctx->d_arena, first, F, dst);
-    } else {
         ++ctx->launches;
-        k_compose<OutT><<<grid_for(V, NT), NT, 0, ctx->stream>>>(ctx->d_ctl, ctx->d_arena, round, dst);
+        k_compose_table<<<grid_for(n, NT), NT, 0, ctx->stream>>>(ctx->d_ctl, ctx->d_arena, first, round, n, F);
+        *last = first - 1;
+        return F;
     }
+    *last = round;
+    return nullptr;
+}
+template <typename OutT>
+static void enqueue_compose(gseg_ctx *ctx, int round, OutT *dst) {
+    const size_t V = (size_t)ctx->w * ctx->h;
+    int last;
+    const u32 *F = compose_table(ctx, round, &last);
+    ++ctx->launches;
+    if (F) k_compose_px<OutT><<<grid_for(V, NT), NT, 0, ctx->stream>>>(ctx->d_ctl, ctx->d_arena, last + 1, F, dst);
+    else k_compose<OutT><<<grid_for(V, NT), NT, 0, ctx->stream>>>(ctx->d_ctl, ctx->d_arena, round, dst);
 }
 
 extern "C" int gseg_label_bytes(const gseg_ctx *ctx, int level) {
@@ -1395,6 +1425,166 @@ extern "C" int gseg_colorize(gseg_ctx *ctx, int level, uint64_t seed, uint8_t *o
     CK(cudaGetLastError());
     if (mem_kind != GSEG_MEM_DEVICE) CK(cudaMemcpyAsync(out, dst, 3 * V, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
+    return GSEG_OK;
+}
+
+// ---- region statistics and pictures (gseg_regions.cuh) ------------------------------------------------------
+// Scratch, all of it free once a run is complete: d_wsel (the composed table of deep levels, as gseg_labels_ex),
+// d_best[0] (the table on its way to host memory, up to (Vmax + 64) / 8 records; larger ones use d_rtab, allocated by
+// GSEG_CAP_REGIONS or on first need), d_labels[1] (host-memory input), d_labels[0] (gseg_render's label image), d_rank
+// (mean colours), d_succ (gseg_render's picture on its way to host memory).  d_attr and the edge lists are left alone:
+// gseg_export_graph / gseg_strip_record still read them after a run.
+static int regions_state(gseg_ctx *ctx, int level, int *round, int *n) {
+    if (!ctx->valid) return fail(ctx, GSEG_E_STATE, "no completed segmentation in this context", cudaSuccess);
+    if (ctx->graph_mode || ctx->strip_labels)
+        return fail(ctx, GSEG_E_STATE, "the last run was an explicit-graph run or a joined strip (no input image)", cudaSuccess);
+    int rc = level_to_round(ctx, level, round);
+    if (rc) return rc;
+    *n = gseg_num_components(ctx, level);
+    return *n < 0 ? *n : GSEG_OK;
+}
+
+// The image the run read: `rgb` as given (host memory is staged in d_labels[1]), or the context's staged input.
+static int regions_input(gseg_ctx *ctx, const uint8_t *rgb, int stride, int kind, const uint8_t **src, long long *sstride) {
+    const int w = ctx->w, h = ctx->h;
+    if (!rgb) {
+        if (!ctx->rgb_staged) return fail(ctx, GSEG_E_STATE, "the run read caller-owned device memory: pass its input", cudaSuccess);
+        *src = ctx->d_rgb + (size_t)3 * w * ctx->halo_top;
+        *sstride = 3LL * w;
+        return GSEG_OK;
+    }
+    if (stride < 3 * w) return fail(ctx, GSEG_E_ARG, "input stride", cudaSuccess);
+    if (kind == GSEG_MEM_DEVICE) { *src = rgb; *sstride = stride; return GSEG_OK; }
+    if (kind != GSEG_MEM_HOST) return fail(ctx, GSEG_E_ARG, "rgb_mem_kind", cudaSuccess);
+    int rc = ensure(ctx, &ctx->d_labels[1], ctx->Vmax + 64); // 4V bytes >= the 3V of the image
+    if (rc) return rc;
+    uint8_t *d = (uint8_t *)ctx->d_labels[1];
+    CK(cudaMemcpy2DAsync(d, (size_t)3 * w, rgb, (size_t)stride, (size_t)3 * w, (size_t)h, cudaMemcpyHostToDevice, ctx->stream));
+    *src = d;
+    *sstride = 3LL * w;
+    return GSEG_OK;
+}
+
+// Enqueue the table of the level ending at `round` (n components) into device memory `table`.  Tier: the block-private
+// shared-memory table when n <= rg_smem_max and it fits, else global atomics.  Shared-memory fields are 32-bit: a block
+// takes at most P = (2^32 - 1) / max(255, w - 1, h - 1) pixels, so no sum of a channel or a coordinate over its pixels
+// can exceed 2^32 - 1 (1080p: P = 2.2 M pixels, far above what a block gets anyway).
+static int regions_enqueue(gseg_ctx *ctx, int round, u32 n, const uint8_t *src, long long sstride, u64 *table) {
+    cudaStream_t s = ctx->stream;
+    const u32 w = (u32)ctx->w, h = (u32)ctx->h;
+    const u32 cpr = (w + RG_K - 1) / RG_K, nch = cpr * h;
+    u32 wide = w - 1 > h - 1 ? w - 1 : h - 1;
+    if (wide < 255u) wide = 255u;
+    const u64 cpb_max = (0xFFFFFFFFull / wide) / RG_K; // chunks per block that keep the shared fields within 32 bits
+    const bool smem = n <= ctx->rg_smem_max && n <= ctx->rg_smem_fit && cpb_max >= 1;
+    u64 grid = (u64)ctx->num_sms * 4u;
+    const u64 gmax = ((u64)nch + NT - 1) / NT; // at least one chunk per thread
+    if (grid > gmax) grid = gmax;
+    if (smem && grid < ((u64)nch + cpb_max - 1) / cpb_max) grid = ((u64)nch + cpb_max - 1) / cpb_max;
+    if (grid < 1) grid = 1;
+    const u32 cpb = (u32)(((u64)nch + grid - 1) / grid);
+    grid = ((u64)nch + cpb - 1) / cpb;
+    mark_end(ctx, s); // the composed table below is not one of the profiled kernels
+    int last;
+    const u32 *F = compose_table(ctx, round, &last);
+    ctx->rg_n = n;
+    mark(ctx, s, "k_regions_init", round);
+    k_regions_init<<<grid_for(n, NT), NT, 0, s>>>(table, n);
+    if (smem) {
+        mark(ctx, s, "k_regions_smem", round);
+        k_regions<true><<<(unsigned)grid, NT, (size_t)n * RG_FIELDS * sizeof(u32), s>>>(ctx->d_ctl, ctx->d_arena, last, F, src,
+                                                                                        sstride, w, h, n, cpb, table);
+    } else {
+        mark(ctx, s, "k_regions_gl", round);
+        k_regions<false><<<(unsigned)grid, NT, 0, s>>>(ctx->d_ctl, ctx->d_arena, last, F, src, sstride, w, h, n, cpb, table);
+    }
+    mark_end(ctx, s);
+    CK(cudaGetLastError());
+    return GSEG_OK;
+}
+
+// Device scratch for a table of n records on its way elsewhere.
+static int regions_scratch(gseg_ctx *ctx, u32 n, u64 **table) {
+    if ((size_t)n * 8 <= ctx->Vmax + 64) { *table = ctx->d_best[0]; return GSEG_OK; }
+    int rc = ensure(ctx, &ctx->d_rtab, 8 * (ctx->Vmax + 64));
+    *table = ctx->d_rtab;
+    return rc;
+}
+
+extern "C" int gseg_regions_async(gseg_ctx *ctx, int level, const uint8_t *rgb, int stride, int rgb_mem_kind, uint64_t *out,
+                                  int64_t cap_records, int mem_kind) {
+    if (!ctx || !out) return GSEG_E_ARG;
+    if (mem_kind != GSEG_MEM_HOST && mem_kind != GSEG_MEM_DEVICE) return GSEG_E_ARG;
+    if (mem_kind == GSEG_MEM_DEVICE && ((uintptr_t)out & 7u)) return fail(ctx, GSEG_E_ARG, "device table not 8-byte aligned", cudaSuccess);
+    int round, n;
+    int rc = regions_state(ctx, level, &round, &n);
+    if (rc) return rc;
+    if (cap_records < n) return fail(ctx, GSEG_E_RANGE, "region table capacity below the component count", cudaSuccess);
+    CK(cudaSetDevice(ctx->device));
+    const uint8_t *src;
+    long long sstride;
+    rc = regions_input(ctx, rgb, stride, rgb_mem_kind, &src, &sstride);
+    if (rc) return rc;
+    u64 *table = (u64 *)out;
+    if (mem_kind != GSEG_MEM_DEVICE && (rc = regions_scratch(ctx, (u32)n, &table)) != 0) return rc;
+    rc = regions_enqueue(ctx, round, (u32)n, src, sstride, table);
+    if (rc) return rc;
+    if (mem_kind != GSEG_MEM_DEVICE) CK(cudaMemcpyAsync(out, table, (size_t)n * 64, cudaMemcpyDeviceToHost, ctx->stream));
+    return n;
+}
+
+extern "C" int gseg_regions(gseg_ctx *ctx, int level, const uint8_t *rgb, int stride, int rgb_mem_kind, uint64_t *out,
+                            int64_t cap_records, int mem_kind) {
+    const int n = gseg_regions_async(ctx, level, rgb, stride, rgb_mem_kind, out, cap_records, mem_kind);
+    if (n < 0) return n;
+    const int rc = gseg_sync(ctx);
+    return rc ? rc : n;
+}
+
+extern "C" int gseg_render(gseg_ctx *ctx, int level, int mode, uint32_t colour, const uint8_t *rgb, int stride, int rgb_mem_kind,
+                           uint8_t *out, int mem_kind) {
+    if (!ctx || !out) return GSEG_E_ARG;
+    if (mode != GSEG_RENDER_MEAN && mode != GSEG_RENDER_OVERLAY && mode != GSEG_RENDER_BOUNDARY) return GSEG_E_ARG;
+    if (mem_kind != GSEG_MEM_HOST && mem_kind != GSEG_MEM_DEVICE) return GSEG_E_ARG;
+    int round, n;
+    int rc = regions_state(ctx, level, &round, &n);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t s = ctx->stream;
+    const u32 w = (u32)ctx->w, h = (u32)ctx->h;
+    const size_t V = (size_t)w * h;
+    const uint8_t *src = nullptr;
+    long long sstride = 0;
+    if (mode != GSEG_RENDER_BOUNDARY && (rc = regions_input(ctx, rgb, stride, rgb_mem_kind, &src, &sstride)) != 0) return rc;
+    const u32 *mean = nullptr;
+    if (mode == GSEG_RENDER_MEAN) {
+        u64 *table;
+        if ((rc = regions_scratch(ctx, (u32)n, &table)) != 0) return rc;
+        if ((rc = regions_enqueue(ctx, round, (u32)n, src, sstride, table)) != 0) return rc;
+        mark(ctx, s, "k_region_means", round);
+        k_region_means<<<grid_for((size_t)n, NT), NT, 0, s>>>(table, (u32)n, ctx->d_rank);
+        mean = ctx->d_rank;
+    }
+    mark_end(ctx, s);
+    enqueue_compose<int>(ctx, round, ctx->d_labels[0]);
+    uint8_t *dst = mem_kind == GSEG_MEM_DEVICE ? out : (uint8_t *)ctx->d_succ; // 4V bytes >= the 3V of a picture
+    const int aligned = ((uintptr_t)dst & 3u) == 0;
+    const int g = grid_for((V + 3) / 4, NT);
+    if (mode == GSEG_RENDER_MEAN) {
+        mark(ctx, s, "k_render_mean", round);
+        k_render<GSEG_RENDER_MEAN_><<<g, NT, 0, s>>>(ctx->d_labels[0], w, h, mean, src, sstride, colour, dst, aligned);
+    } else if (mode == GSEG_RENDER_OVERLAY) {
+        mark(ctx, s, "k_render_overlay", round);
+        k_render<GSEG_RENDER_OVERLAY_><<<g, NT, 0, s>>>(ctx->d_labels[0], w, h, mean, src, sstride, colour, dst, aligned);
+    } else {
+        mark(ctx, s, "k_render_boundary", round);
+        k_render<GSEG_RENDER_BOUNDARY_><<<g, NT, 0, s>>>(ctx->d_labels[0], w, h, mean, src, sstride, colour, dst, aligned);
+    }
+    mark_end(ctx, s);
+    CK(cudaGetLastError());
+    if (mem_kind != GSEG_MEM_DEVICE)
+        CK(cudaMemcpyAsync(out, dst, V * (mode == GSEG_RENDER_BOUNDARY ? 1 : 3), cudaMemcpyDeviceToHost, s));
+    CK(cudaStreamSynchronize(s));
     return GSEG_OK;
 }
 
@@ -1830,6 +2020,15 @@ static void algo_bytes(const gseg_ctx *c, const char *name, int r, double *algo,
     else if (!strcmp(name, "k_edges")) { a = 12 * E + 8 * E + 12 * En + 8 * Vn + (sp ? 32 * En : 0); s = 12 * E + 4 * V + 12 * En + 8 * Vn + (sp ? 16 * Vn : 0); }
     else if (!strcmp(name, "k_means")) a = s = 32 * Vn + 16 * Vn;
     else if (!strcmp(name, "k_page_scan")) a = s = 8.0 * h->stPages[r];
+    // region statistics (gseg_regions.cuh): the input (3 V) and the round-0 map of the fused label chase (4 V) in, the
+    // table (64 B per component) out; later maps and the composed table are gathers of few components (cached)
+    else if (!strcmp(name, "k_regions_smem") || !strcmp(name, "k_regions_gl")) a = s = 3 * V0 + 4 * V0 + 64.0 * c->rg_n;
+    else if (!strcmp(name, "k_regions_init")) a = s = 64.0 * c->rg_n;
+    else if (!strcmp(name, "k_region_means")) a = s = 32.0 * c->rg_n + 4.0 * c->rg_n;
+    // pictures: the label image in (4 V; the stencil's neighbours are the same array), the picture out
+    else if (!strcmp(name, "k_render_mean")) { a = 4 * V0 + 4 * V0 + 3 * V0; s = 4 * V0 + 4.0 * c->rg_n + 3 * V0; }
+    else if (!strcmp(name, "k_render_overlay")) a = s = 4 * V0 + 3 * V0 + 3 * V0;
+    else if (!strcmp(name, "k_render_boundary")) a = s = 4 * V0 + V0;
     *algo = a; *strict = s;
 }
 

@@ -14,6 +14,9 @@
 //     --conn 4|8                     grid connectivity (default 8, as in `segment`)
 //     --level L                      hierarchy level to write (hier/superpix; default last)
 //     --labels FILE                  also write the label image as raw little-endian int32, row-major
+//     --regions FILE                 also write the region table (gseg_regions: 8 little-endian uint64 per component)
+//     --render random|mean|overlay   output picture: random colour per component (default), each region's mean colour,
+//                                    or the input with the region boundaries in red (gseg_render)
 //     --synth WxH:SEED               ignore input.ppm, segment the deterministic synthetic image
 //     --iters N                      timing loop: N runs after 2 warm-ups, mean +- std (excludes I/O)
 //     --device D                     CUDA device ordinal
@@ -22,7 +25,9 @@
 //   gseg --batch IN_DIR OUT_DIR [options] sigma k min_size
 //     every image file of IN_DIR (PPM/PGM/PNG, or JPEG decoded on the GPU) through the batch pipeline gseg_pool_*
 //     (--contexts S contexts in flight, default 8); writes OUT_DIR/<name>.png (random colours per component, same
-//     colours as the single-image mode) and prints one "name: got N components" line per image plus the throughput
+//     colours as the single-image mode) and prints one "name: got N components" line per image plus the throughput;
+//     --render mean: the jobs return the region table with the labels (GSEG_OUT_REGIONS) and the mean-colour picture is
+//     painted on the host from it, without a second pass on the device
 //   gseg --convert input output      file conversion only (no GPU): exercises the readers/writers
 #include <dirent.h>
 
@@ -50,9 +55,16 @@ static inline void label_colour(uint64_t seed, uint32_t label, uint8_t *rgb) {
     const uint64_t h = sm64(sm64(seed ^ ((uint64_t)label * 0xD6E8FEB86659FD93ull)) + 3);
     rgb[0] = (uint8_t)(h & 255); rgb[1] = (uint8_t)((h >> 8) & 255); rgb[2] = (uint8_t)((h >> 16) & 255);
 }
+// Rounded mean colour of record c of a region table: (sum + count / 2) / count, as gseg_render(GSEG_RENDER_MEAN).
+static inline void mean_colour(const uint64_t *table, uint32_t c, uint8_t *rgb) {
+    const uint64_t *t = table + 8 * (size_t)c, n = t[0] ? t[0] : 1;
+    for (int k = 0; k < 3; ++k) rgb[k] = (uint8_t)((t[1 + k] + n / 2) / n);
+}
+
+#define RENDER_RANDOM (-1)
 
 // gseg --batch IN_DIR OUT_DIR: the reference's loop over a directory of images, through the batch pipeline.
-static int run_batch(const char *in_dir, const char *out_dir, const gseg_params &p, int level, int device, int contexts) {
+static int run_batch(const char *in_dir, const char *out_dir, const gseg_params &p, int level, int device, int contexts, int render) {
     std::vector<std::string> names;
     if (DIR *d = opendir(in_dir)) {
         while (dirent *e = readdir(d)) {
@@ -108,7 +120,13 @@ static int run_batch(const char *in_dir, const char *out_dir, const gseg_params 
         }
         j.w = it.w; j.h = it.h; j.stride_bytes = 3 * it.w; j.mem_kind = GSEG_MEM_HOST; j.params = p;
         j.out_mode = GSEG_OUT_LABELS; j.level = p.variant == GSEG_FELZ ? -1 : level; j.elem_bytes = 4; j.out_mem_kind = GSEG_MEM_HOST;
-        j.out = gseg_host_alloc(V * 4); j.out_capacity = V * 4;
+        j.out_capacity = V * 4;
+        if (render == GSEG_RENDER_MEAN) { // labels, then the table at the next 64-byte boundary; a FELZ component has >= min_size pixels
+            const size_t ncap = p.variant == GSEG_FELZ && p.min_size > 1 ? (V + p.min_size - 1) / p.min_size : V;
+            j.out_mode = GSEG_OUT_REGIONS;
+            j.out_capacity = ((V * 4 + 63) & ~(size_t)63) + 64 * ncap;
+        }
+        j.out = gseg_host_alloc(j.out_capacity);
         if (!j.out) { fprintf(stderr, "gseg: pinned allocation failed\n"); return 1; }
         pinned.push_back(j.out);
     }
@@ -122,7 +140,12 @@ static int run_batch(const char *in_dir, const char *out_dir, const gseg_params 
         mpix += V / 1e6;
         std::vector<uint8_t> out(V * 3);
         const int32_t *lab = (const int32_t *)jobs[i].out;
-        for (size_t q = 0; q < V; ++q) label_colour(1, (uint32_t)lab[q], &out[3 * q]);
+        if (render == GSEG_RENDER_MEAN) {
+            const uint64_t *table = (const uint64_t *)((const uint8_t *)jobs[i].out + res[i].offsets[1]);
+            for (size_t q = 0; q < V; ++q) mean_colour(table, (uint32_t)lab[q], &out[3 * q]);
+        } else {
+            for (size_t q = 0; q < V; ++q) label_colour(1, (uint32_t)lab[q], &out[3 * q]);
+        }
         const std::string stem = names[i].substr(0, names[i].rfind('.'));
         const std::string path = std::string(out_dir) + "/" + stem + ".png";
         if (!gsegio::write_image(path.c_str(), out.data(), res[i].w, res[i].h)) { fprintf(stderr, "gseg: cannot write %s\n", path.c_str()); return 1; }
@@ -136,9 +159,11 @@ static int run_batch(const char *in_dir, const char *out_dir, const gseg_params 
 
 static int usage() {
     fprintf(stderr,
-            "usage: gseg [--variant felz|hier|superpix] [--conn 4|8] [--level L] [--labels FILE]\n"
-            "            [--synth WxH:SEED] [--iters N] [--device D] [--host-loop] [--tail E,V] sigma k min_size input.{ppm,pgm,png,jpg} output.{ppm,png}\n"
-            "       gseg --batch IN_DIR OUT_DIR [--contexts S] [--variant ...] [--conn 4|8] [--level L] [--device D] sigma k min_size\n"
+            "usage: gseg [--variant felz|hier|superpix] [--conn 4|8] [--level L] [--labels FILE] [--regions FILE]\n"
+            "            [--render random|mean|overlay] [--synth WxH:SEED] [--iters N] [--device D] [--host-loop] [--tail E,V]\n"
+            "            sigma k min_size input.{ppm,pgm,png,jpg} output.{ppm,png}\n"
+            "       gseg --batch IN_DIR OUT_DIR [--contexts S] [--variant ...] [--conn 4|8] [--level L] [--render random|mean]\n"
+            "            [--device D] sigma k min_size\n"
             "       gseg --convert input output\n");
     return 2;
 }
@@ -162,7 +187,8 @@ int main(int argc, char **argv) {
     int contexts = 8;
     const char *batch_in = nullptr, *batch_out = nullptr;
     unsigned long long sseed = 0;
-    const char *labels_path = nullptr;
+    const char *labels_path = nullptr, *regions_path = nullptr;
+    int render = RENDER_RANDOM;
     std::vector<const char *> pos;
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
@@ -179,6 +205,14 @@ int main(int argc, char **argv) {
         } else if (a == "--conn") p.connectivity = atoi(need("--conn"));
         else if (a == "--level") level = atoi(need("--level"));
         else if (a == "--labels") labels_path = need("--labels");
+        else if (a == "--regions") regions_path = need("--regions");
+        else if (a == "--render") {
+            std::string v = need("--render");
+            if (v == "random") render = RENDER_RANDOM;
+            else if (v == "mean") render = GSEG_RENDER_MEAN;
+            else if (v == "overlay") render = GSEG_RENDER_OVERLAY;
+            else return usage();
+        }
         else if (a == "--iters") iters = atoi(need("--iters"));
         else if (a == "--device") device = atoi(need("--device"));
         else if (a == "--host-loop") p.flags |= GSEG_FLAG_HOST_LOOP;
@@ -191,9 +225,9 @@ int main(int argc, char **argv) {
         else pos.push_back(argv[i]);
     }
     if (batch_in) {
-        if (pos.size() != 3 || contexts < 1 || contexts > 64) return usage();
+        if (pos.size() != 3 || contexts < 1 || contexts > 64 || render == GSEG_RENDER_OVERLAY || regions_path) return usage();
         p.sigma = (float)atof(pos[0]); p.k = (float)atof(pos[1]); p.min_size = atoi(pos[2]);
-        return run_batch(batch_in, batch_out, p, level, device, contexts);
+        return run_batch(batch_in, batch_out, p, level, device, contexts, render);
     }
     if (pos.size() != 5) return usage();
     p.sigma = (float)atof(pos[0]);
@@ -259,8 +293,14 @@ int main(int argc, char **argv) {
     }
     const int ncomp = gseg_num_components(ctx, p.variant == GSEG_FELZ ? -1 : level);
     std::vector<uint8_t> out((size_t)w * h * 3);
-    rc = gseg_colorize(ctx, p.variant == GSEG_FELZ ? -1 : level, 1, out.data(), GSEG_MEM_HOST);
-    if (rc) { fprintf(stderr, "gseg: gseg_colorize: %s\n", gseg_strerror(rc)); return 1; }
+    const int olevel = p.variant == GSEG_FELZ ? -1 : level;
+    if (render == RENDER_RANDOM) {
+        rc = gseg_colorize(ctx, olevel, 1, out.data(), GSEG_MEM_HOST);
+        if (rc) { fprintf(stderr, "gseg: gseg_colorize: %s\n", gseg_strerror(rc)); return 1; }
+    } else { // the input the context staged (the last gseg_segment read host memory)
+        rc = gseg_render(ctx, olevel, render, 0xFF0000u, nullptr, 0, GSEG_MEM_HOST, out.data(), GSEG_MEM_HOST);
+        if (rc) { fprintf(stderr, "gseg: gseg_render: %s (%s)\n", gseg_strerror(rc), gseg_last_error(ctx)); return 1; }
+    }
     if (!gsegio::write_image(out_path, out.data(), w, h)) { fprintf(stderr, "gseg: cannot write %s\n", out_path); return 1; }
     if (labels_path) {
         std::vector<int32_t> lab((size_t)w * h);
@@ -269,6 +309,17 @@ int main(int argc, char **argv) {
         FILE *f = fopen(labels_path, "wb");
         if (!f || fwrite(lab.data(), sizeof(int32_t), lab.size(), f) != lab.size()) {
             fprintf(stderr, "gseg: cannot write %s\n", labels_path);
+            return 1;
+        }
+        fclose(f);
+    }
+    if (regions_path) {
+        std::vector<uint64_t> table((size_t)ncomp * 8);
+        rc = gseg_regions(ctx, olevel, nullptr, 0, GSEG_MEM_HOST, table.data(), ncomp, GSEG_MEM_HOST);
+        if (rc < 0) { fprintf(stderr, "gseg: gseg_regions: %s (%s)\n", gseg_strerror(rc), gseg_last_error(ctx)); return 1; }
+        FILE *f = fopen(regions_path, "wb");
+        if (!f || fwrite(table.data(), sizeof(uint64_t), table.size(), f) != table.size()) {
+            fprintf(stderr, "gseg: cannot write %s\n", regions_path);
             return 1;
         }
         fclose(f);

@@ -28,6 +28,9 @@ struct Rec {
     gseg_pool_result res;
     int slot;
     bool running;       // the segmentation has been enqueued but not waited for
+    const uint8_t *rgb; // GSEG_OUT_REGIONS: the device image the job read (nullptr: the context staged it itself)
+    int rgb_stride;
+    int stage_b;        // ... which is pool staging buffer stage[stage_b] (-1: it is not)
     cudaEvent_t ev;     // completion of the output copy (nullptr: nothing was enqueued)
 };
 
@@ -44,6 +47,11 @@ struct gseg_pool {
     std::vector<uint8_t *> stage;      // [2 * S]
     std::vector<cudaEvent_t> stage_ev; // [2 * S]
     std::vector<int> stage_next;       // per context: which of its two buffers the next job takes
+    // 1: a GSEG_OUT_REGIONS job's statistics kernel reads stage[b] on the context's stream after its segmentation was
+    // waited for, and stage_ev[b] was re-recorded behind it there: the next write into stage[b] (host copy or JPEG decode,
+    // on the copy stream) waits for that event first.  Without it, jpeg_prefetch would decode job t + 2S into the buffer
+    // while job t's k_regions (enqueued by retire in the submit of job t + S) may still be reading it.
+    std::vector<int> stage_read;       // [2 * S]
     // JPEG jobs: the decode of a context's NEXT job (in-house kernels, on the copy stream, into the free staging buffer) is
     // enqueued as soon as the current one has been submitted -- a whole pipeline turn ahead (gseg_pool_run knows the job)
     struct Pref { const void *input; size_t bytes; int w, h, b; bool valid; };
@@ -88,6 +96,7 @@ extern "C" int gseg_pool_create(gseg_pool **out, int device, int max_w, int max_
                 if (cudaMalloc((void **)&d, p->stage_bytes + 64) != cudaSuccess || cudaEventCreateWithFlags(&e, cudaEventDisableTiming) != cudaSuccess) rc = GSEG_E_CUDA;
                 p->stage.push_back(d);
                 p->stage_ev.push_back(e);
+                p->stage_read.push_back(0);
             }
             if (caps) rc = gseg_reserve(c, caps);
             // several contexts share the SMs: size every grid for 2 resident blocks per SM so that kernels of
@@ -135,6 +144,13 @@ extern "C" const char *gseg_pool_last_error(const gseg_pool *p) { return p ? p->
 
 // The job's segmentation is complete on the device: read what the host needs to know, enqueue the output copy
 // on the context's stream and mark its end with an event.  The context is free for its next job afterwards.
+// A write into stage[b] on the copy stream of `slot` is about to be enqueued: order it behind a reader retire left.
+static cudaError_t stage_claim(gseg_pool *p, int slot, int b) {
+    if (!p->stage_read[(size_t)b]) return cudaSuccess;
+    p->stage_read[(size_t)b] = 0;
+    return cudaStreamWaitEvent(p->copy_stream[(size_t)slot], p->stage_ev[(size_t)b], 0);
+}
+
 static void retire(gseg_pool *p, Rec &r) {
     gseg_ctx *c = p->ctx[(size_t)r.slot];
     r.running = false;
@@ -152,6 +168,23 @@ static void retire(gseg_pool *p, Rec &r) {
         if (!r.job.out || V * (size_t)eb > r.job.out_capacity) { res.status = GSEG_E_RANGE; return; }
         rc = gseg_labels_ex_async(c, r.job.level, r.job.out, eb, r.job.out_mem_kind);
         res.elem_bytes = eb; res.out_bytes = (int64_t)(V * (size_t)eb);
+    } else if (r.job.out_mode == GSEG_OUT_REGIONS) {
+        const int need = gseg_label_bytes(c, r.job.level);
+        const int eb = r.job.elem_bytes ? r.job.elem_bytes : need;
+        const size_t off = (V * (size_t)eb + 63) & ~(size_t)63, end = off + (size_t)res.n_components * 64;
+        if (!r.job.out || end > r.job.out_capacity) { res.status = GSEG_E_RANGE; return; }
+        rc = gseg_labels_ex_async(c, r.job.level, r.job.out, eb, r.job.out_mem_kind);
+        if (!rc) {
+            rc = gseg_regions_async(c, r.job.level, r.rgb, r.rgb_stride, GSEG_MEM_DEVICE, (uint64_t *)((uint8_t *)r.job.out + off),
+                                    res.n_components, r.job.out_mem_kind);
+            if (rc >= 0) rc = GSEG_OK;
+        }
+        if (!rc && r.stage_b >= 0) { // the staging buffer is read until here: see gseg_pool::stage_read
+            cudaEventRecord(p->stage_ev[(size_t)r.stage_b], (cudaStream_t)gseg_get_stream(c));
+            p->stage_read[(size_t)r.stage_b] = 1;
+        }
+        res.elem_bytes = eb; res.offsets[0] = 0; res.offsets[1] = (int64_t)off; res.offsets[2] = (int64_t)end;
+        res.out_bytes = (int64_t)end;
     } else if (r.job.out_mode == GSEG_OUT_HIERARCHY) {
         rc = gseg_hierarchy_async(c, (uint32_t *)r.job.out, (int64_t)(r.job.out_capacity / 4), res.offsets, GSEG_POOL_MAXLEVELS + 1,
                                   r.job.out_mem_kind);
@@ -175,6 +208,7 @@ static int jpeg_prefetch(gseg_pool *p, int slot, const gseg_pool_job *job) {
     gseg_ctx *c = p->ctx[(size_t)slot];
     const int b = 2 * slot + p->stage_next[(size_t)slot];
     int w = 0, h = 0;
+    if (stage_claim(p, slot, b) != cudaSuccess) { cudaGetLastError(); return GSEG_E_CUDA; }
     const int rc = gseg_jpeg_decode_async(c, job->input, job->jpeg_bytes, p->stage[(size_t)b], p->stage_bytes, p->copy_stream[(size_t)slot], &w, &h);
     if (rc) return rc;
     if (cudaEventRecord(p->stage_ev[(size_t)b], p->copy_stream[(size_t)slot]) != cudaSuccess) { cudaGetLastError(); return GSEG_E_CUDA; }
@@ -185,7 +219,7 @@ static int jpeg_prefetch(gseg_pool *p, int slot, const gseg_pool_job *job) {
 
 extern "C" int gseg_pool_submit(gseg_pool *p, const gseg_pool_job *job, int64_t *ticket) {
     if (!p || !job || !job->input) return GSEG_E_ARG;
-    if (job->out_mode < GSEG_OUT_NONE || job->out_mode > GSEG_OUT_HIERARCHY) return GSEG_E_ARG;
+    if (job->out_mode < GSEG_OUT_NONE || job->out_mode > GSEG_OUT_REGIONS) return GSEG_E_ARG;
     if (job->elem_bytes != 0 && job->elem_bytes != 1 && job->elem_bytes != 2 && job->elem_bytes != 4) return GSEG_E_ARG;
     if (job->out_mode != GSEG_OUT_NONE && (!job->out || (job->out_mem_kind != GSEG_MEM_HOST && job->out_mem_kind != GSEG_MEM_DEVICE)))
         return GSEG_E_ARG;
@@ -198,7 +232,8 @@ extern "C" int gseg_pool_submit(gseg_pool *p, const gseg_pool_job *job, int64_t 
         (size_t)job->w * (size_t)job->h * 3 <= p->stage_bytes) {
         const int b = 2 * slot + p->stage_next[(size_t)slot];
         const size_t row = (size_t)3 * job->w, stride = job->stride_bytes ? (size_t)job->stride_bytes : row;
-        cudaError_t e = stride == row
+        cudaError_t e = stage_claim(p, slot, b);
+        if (e == cudaSuccess) e = stride == row
                             ? cudaMemcpyAsync(p->stage[(size_t)b], job->input, row * job->h, cudaMemcpyHostToDevice, p->copy_stream[(size_t)slot])
                             : cudaMemcpy2DAsync(p->stage[(size_t)b], row, job->input, stride, row, (size_t)job->h, cudaMemcpyHostToDevice,
                                                 p->copy_stream[(size_t)slot]);
@@ -226,7 +261,10 @@ extern "C" int gseg_pool_submit(gseg_pool *p, const gseg_pool_job *job, int64_t 
             if (r.running && r.slot == slot) { retire(p, r); break; }
     Rec r;
     memset(&r, 0, sizeof(r));
-    r.job = *job; r.slot = slot; r.running = true; r.ev = nullptr;
+    r.job = *job; r.slot = slot; r.running = true; r.ev = nullptr; r.stage_b = -1;
+    if (!job->jpeg_bytes && job->mem_kind == GSEG_MEM_DEVICE) { // caller-owned device input (nullptr: the context stages it)
+        r.rgb = (const uint8_t *)job->input; r.rgb_stride = job->stride_bytes ? job->stride_bytes : 3 * job->w;
+    }
     r.res.ticket = p->next_ticket; r.res.user = job->user; r.res.out = job->out; r.res.w = job->w; r.res.h = job->h;
     int rc;
     if (job->jpeg_bytes && !dev_input) {
@@ -239,6 +277,7 @@ extern "C" int gseg_pool_submit(gseg_pool *p, const gseg_pool_job *job, int64_t 
         cudaStreamWaitEvent((cudaStream_t)gseg_get_stream(c), p->stage_ev[(size_t)b], 0);
         rc = gseg_segment_async(c, dev_input, w, h, 3 * w, GSEG_MEM_DEVICE, &job->params);
         r.res.w = w; r.res.h = h;
+        r.rgb = dev_input; r.rgb_stride = 3 * w; r.stage_b = b;
     } else {
         rc = gseg_segment_async(c, (const uint8_t *)job->input, job->w, job->h, job->stride_bytes ? job->stride_bytes : 3 * job->w,
                                 job->mem_kind, &job->params);

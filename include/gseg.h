@@ -114,6 +114,8 @@ void gseg_destroy(gseg_ctx *ctx);
 #define GSEG_CAP_WIDE_SIGMA 2u /* intermediate plane of the general blur (more than 8 one-sided taps) */
 #define GSEG_CAP_LEVELS 4u     /* second staging buffer of gseg_labels_all / gseg_colorize to host memory */
 #define GSEG_CAP_JPEG 8u       /* buffers of the in-house JPEG decoder (staged file, coefficients, sample planes) */
+#define GSEG_CAP_REGIONS 16u   /* gseg_regions / gseg_render scratch: a table of 64 bytes per pixel (host output of tables
+                                  with more than (max_w*max_h + 64)/8 records) and the staging of host-memory input */
 int gseg_reserve(gseg_ctx *ctx, uint32_t caps);
 
 /* Pinned host memory for inputs/outputs of the asynchronous calls (cudaHostAlloc behind a plain pointer, so a
@@ -202,6 +204,26 @@ int gseg_labels_all(gseg_ctx *ctx, int32_t *out, int max_levels, int mem_kind);
 
 /* Replaces: random colour table + colour image (cuRAND, Report p4 s3.2.3).  out: w*h*3 bytes. */
 int gseg_colorize(gseg_ctx *ctx, int level, uint64_t seed, uint8_t *out_rgb, int mem_kind);
+
+/* Per-component statistics of `level` (same level rules as gseg_labels_ex; component c = dense label c):
+ * out[8*c + 0..7] = count, sum r, sum g, sum b (the INPUT image's 8-bit channels), sum x, sum y,
+ * x0 | y0 << 32 (bounding-box minimum, inclusive), x1 | y1 << 32 (maximum, inclusive) -- n = gseg_num_components(level)
+ * records of 64 bytes, all integers (DESIGN.md section 2 item 10).  The input is `rgb` (stride_bytes per row, host or
+ * device memory as rgb_mem_kind says), or with rgb == NULL the image the context staged (host input or JPEG;
+ * GSEG_E_STATE when the run read caller-owned device memory).  GSEG_E_STATE after an explicit-graph run or a joined
+ * strip, GSEG_E_RANGE when cap_records < n, GSEG_E_ARG for device output that is not 8-byte aligned.  Returns n. */
+int gseg_regions_async(gseg_ctx *ctx, int level, const uint8_t *rgb, int stride_bytes, int rgb_mem_kind, uint64_t *out,
+                       int64_t cap_records, int mem_kind);
+int gseg_regions(gseg_ctx *ctx, int level, const uint8_t *rgb, int stride_bytes, int rgb_mem_kind, uint64_t *out,
+                 int64_t cap_records, int mem_kind); /* blocking form */
+
+/* Pictures of `level` (blocking).  A boundary pixel has at least one 4-neighbour inside the image with another label.
+ * MEAN and OVERLAY read the input like gseg_regions (rgb == NULL: the staged image); BOUNDARY ignores rgb. */
+#define GSEG_RENDER_MEAN 0     /* every pixel = its region's rounded mean colour (sum + count/2) / count; out: w*h*3 bytes */
+#define GSEG_RENDER_OVERLAY 1  /* input pixels, boundary pixels set to `colour` (0xRRGGBB); out: w*h*3 bytes             */
+#define GSEG_RENDER_BOUNDARY 2 /* 1 byte per pixel: 1 = boundary pixel, 0 = not; out: w*h bytes                           */
+int gseg_render(gseg_ctx *ctx, int level, int mode, uint32_t colour, const uint8_t *rgb, int stride_bytes, int rgb_mem_kind,
+                uint8_t *out, int mem_kind);
 
 /* Round-0 edge weights in edge-index order idx = d*w*h + (y*w+x), d in 0..D-1, D = 2 (E,S) or 4 (E,S,SE,NE);
  * +inf where the edge does not exist (SUPERPIX: the static edge strength).  For the 1e-6 check. */
@@ -338,6 +360,9 @@ long long gseg_compaction_count(const gseg_ctx *ctx);
 #define GSEG_OUT_NONE 0      /* nothing leaves the context (results stay there until its next job) */
 #define GSEG_OUT_LABELS 1    /* label image of `level`; elem_bytes 0 = the narrowest lossless type, else 1 / 2 / 4 */
 #define GSEG_OUT_HIERARCHY 2 /* the stored hierarchy (gseg_hierarchy): level-0 labels + one map per further level */
+#define GSEG_OUT_REGIONS 3   /* label image of `level` as GSEG_OUT_LABELS, then at the next 64-byte-aligned offset the region
+                                table (gseg_regions) of the job's input: offsets[0] = 0, offsets[1] = the table's byte offset,
+                                offsets[2] = out_bytes = the end */
 #define GSEG_POOL_MAXLEVELS 64
 typedef struct gseg_pool gseg_pool;
 typedef struct gseg_pool_job {
