@@ -18,7 +18,7 @@
 //            cooperative 32-ary search, partial minima meet in a 64-bit atomicMin on the run's first element
 //   mark     the winner of every run is flagged by its list position; the per-component minima are reset
 //   compact  ordered compaction of the flagged edges back into the (now dense) paged list
-//   finish   page table + per-component minimum of the next round (segmented warp minima, as k_graph_init)
+//   finish   page table + per-component minimum of the next round (seed_dense_pages, as k_graph_init)
 //
 // Result: unchanged by construction for static weights (FELZ, HIER): the minimum over a set of parallel edges
 // is the minimum over the per-pair minima, and the compaction keeps the list order, i.e. the tie-break.  The
@@ -219,27 +219,17 @@ __global__ void __launch_bounds__(1024) k_dd_compact(GsegCtl *ctl, GsegBufs B, D
 // edge and page counts.
 __global__ void __launch_bounds__(NT) k_dd_finish(GsegCtl *ctl, GsegBufs B, DedupDev *dd) {
     if (!dd->sort.active) return;
-    const RoundState st = load_state(ctl);
-    const int cur = st.round & 1, lane = threadIdx.x & 31;
     const u32 E = dd->kept, P = (E + GSEG_PAGE - 1u) / GSEG_PAGE;
-    for (u32 g = blockIdx.x * (NT / 32) + (threadIdx.x >> 5); g < P; g += gridDim.x * (NT / 32)) {
-        if (lane == 0) { B.pcnt[cur][g] = min(GSEG_PAGE, E - g * GSEG_PAGE); B.poff[cur][g] = g * GSEG_PAGE; }
-#pragma unroll
-        for (int j = 0; j < (int)(GSEG_PAGE / 32); ++j) {
-            const u32 e = g * GSEG_PAGE + 32u * j + lane;
-            const bool act = e < E;
-            uint2 ab = make_uint2(0u, 0u);
-            u32 wv = 0u;
-            if (act) { ab = B.eab[cur][e]; wv = B.ew[cur][e]; }
-            warp_run_min<false, 32>(B.best[cur], ab.x, wv, e, act, 0xFFFFFFFFu);
-            warp_run_min<false, 32>(B.best[cur], ab.y, wv, e, act, 0xFFFFFFFFu);
-        }
-    }
+    // the side as a template argument, and the round state read only where it is needed, keep this kernel at the
+    // registers of the seeding loop (32, as k_graph_init)
+    if (load_state(ctl).round & 1) seed_dense_pages<1>(B, E, P);
+    else seed_dense_pages<0>(B, E, P);
     // the state is read by the kernels AFTER this one; nobody in this kernel reads E or P from it
     __syncthreads();
     if (threadIdx.x == 0) {
         __threadfence();
         if (atomicAdd(&ctl->doneE, 1u) == gridDim.x - 1u) {
+            const RoundState st = load_state(ctl);
             ctl->doneE = 0;
             ctl->ticketE = 0; // the compaction's tickets; the next user (k_page_scan) expects zero
             ctl->stDedupIn[st.round] = st.E; ctl->stDedupOut[st.round] = E;

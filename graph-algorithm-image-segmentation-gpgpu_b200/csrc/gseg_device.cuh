@@ -240,48 +240,6 @@ __device__ __forceinline__ u32 block_ordered_offset(u32 warp_total, u32 btile, u
 
 __device__ __forceinline__ u64 make_key(u32 wbits, u32 idx) { return ((u64)wbits << 32) | (u64)idx; }
 
-// Segmented min-edge selection (SURVEY.md section 8a row a4) by warp shuffles: consecutive lanes that
-// hold edges of the same component `id` form a run; a fixed 5-step segmented min leaves the run's
-// minimum key in its first lane, which alone issues the 64-bit atomicMin.  Edge lists are in
-// edge-index order, so a component's edges come in long runs (a row segment of a component, a stretch
-// of boundary between two components) and the number of atomics falls with the run length.
-// `pos` MUST increase with the lane index (it is the edge's position in the output list), so among
-// equal weights the lower lane already holds the minimum.  All 32 lanes must call.
-template <bool FILTER, int WINDOW>
-__device__ __forceinline__ void warp_run_min(u64 *best, u32 id, u32 kb, u32 pos, bool act, u32 cur_hi) {
-    const int lane = threadIdx.x & 31;
-    const u32 pid = __shfl_up_sync(0xFFFFFFFFu, id, 1);
-    const u32 actm = __ballot_sync(0xFFFFFFFFu, act);
-    const bool head = lane == 0 || pid != id || !((actm >> (lane - 1)) & 1u);
-    const u32 heads = __ballot_sync(0xFFFFFFFFu, head || !act);
-    if (!act) kb = 0xFFFFFFFFu;
-    // lanes [lane, end) belong to this lane's run, end = next head above this lane
-    const u32 above = heads & ~((2u << lane) - 1u);
-    int end = above ? __ffs(above) - 1 : 32;
-    bool lead = head;
-    if (WINDOW < 32) {
-        // early rounds: runs are short, so reduce inside windows of WINDOW lanes of a run (log2(WINDOW) steps
-        // instead of 5) and let every window issue its own atomic
-        const int start = 31 - __clz(heads & ((2u << lane) - 1u)); // first lane of this lane's run
-        const int wstart = start + ((lane - start) & ~(WINDOW - 1));
-        lead = lane == wstart;
-        end = min(end, wstart + WINDOW);
-    }
-#pragma unroll
-    for (int o = 1; o < WINDOW; o <<= 1) {
-        const u32 okb = __shfl_down_sync(0xFFFFFFFFu, kb, o);
-        const u32 opos = __shfl_down_sync(0xFFFFFFFFu, pos, o);
-        if (lane + o < end && okb < kb) { kb = okb; pos = opos; }
-    }
-    if (lead && act) {
-        const u64 key = make_key(kb, pos);
-        // FILTER (components with many edges each): the running minimum only ever decreases, so a key whose
-        // weight is above the weight read earlier (cur_hi: the high word of best[id], prefetched for a whole
-        // tile at once) can never win; skipping it spares the L2 a same-address atomic
-        if (!FILTER || kb <= cur_hi) atomicMin(best + id, key);
-    }
-}
-
 // Rows in which no two neighbouring surviving edges share an end on the same side (every run has length one): the shuffle
 // minima would reduce nothing.  What such rows do have -- they are the stretches of the list that come from direction-E
 // grid edges: a row of the image crosses components A|B|C|..., giving edges (A,B), (B,C), ... -- is that the RIGHT end of
@@ -305,9 +263,15 @@ __device__ __forceinline__ void warp_chain_min(u64 *best, u32 a, u32 b, u32 kb, 
 #endif
 }
 
-// Both ends of a row of edges at once: the two segmented minima are independent dependency chains, so
-// interleaving their shuffles halves the latency of the row (these kernels run few warps per SM in late
+// Segmented min-edge selection (SURVEY.md section 8a row a4) by warp shuffles, both ends of a row of edges at once:
+// consecutive lanes that hold edges of the same component form a run; a fixed 5-step segmented min leaves the run's
+// minimum key in its first lane, which alone issues the 64-bit atomicMin.  Edge lists are in edge-index order, so a
+// component's edges come in long runs (a row segment of a component, a stretch of boundary between two components) and
+// the number of atomics falls with the run length.  The two segmented minima (ends ida, idb) are independent dependency
+// chains, so interleaving their shuffles halves the latency of the row (these kernels run few warps per SM in late
 // rounds and are bound by exactly this chain).
+// `pos` MUST increase with the lane index (it is the edge's position in the output list), so among
+// equal weights the lower lane already holds the minimum.  All 32 lanes must call.
 template <bool FILTER, int WINDOW>
 __device__ __forceinline__ void warp_run_min2(u64 *best, u32 ida, u32 idb, u32 kb, u32 pos, bool act, u32 hia, u32 hib,
                                               u32 *sfilter = nullptr) {
@@ -327,6 +291,8 @@ __device__ __forceinline__ void warp_run_min2(u64 *best, u32 ida, u32 idb, u32 k
     int enda = abva ? __ffs(abva) - 1 : 32, endb = abvb ? __ffs(abvb) - 1 : 32;
     bool leada = heada, leadb = headb;
     if (WINDOW < 32) {
+        // early rounds: runs are short, so reduce inside windows of WINDOW lanes of a run (log2(WINDOW) steps
+        // instead of 5) and let every window issue its own atomic
         const int sa = 31 - __clz(headsa & lmask), sb = 31 - __clz(headsb & lmask);
         const int wa = sa + ((lane - sa) & ~(WINDOW - 1)), wb = sb + ((lane - sb) & ~(WINDOW - 1));
         leada = lane == wa; leadb = lane == wb;
@@ -349,6 +315,9 @@ __device__ __forceinline__ void warp_run_min2(u64 *best, u32 ida, u32 idb, u32 k
         return;
     }
 #ifndef GSEG_EXP_NOATOMIC
+    // FILTER (components with many edges each): the running minimum only ever decreases, so a key whose weight is
+    // above the weight read earlier (hia, hib: the high words of best[ida], best[idb], prefetched for a whole tile at
+    // once) can never win; skipping it spares the L2 a same-address atomic
     if (leada && act && (!FILTER || ka <= hia)) atomicMin(best + ida, make_key(ka, qa));
     if (leadb && act && (!FILTER || kbb <= hib)) atomicMin(best + idb, make_key(kbb, qb));
 #else

@@ -25,6 +25,7 @@
 // are bit-identical to the CPU oracle and the total edge order (weight bits, edge index) is too.
 #pragma once
 #include <cooperative_groups.h>
+#include <type_traits>
 
 #include "gseg_device.cuh"
 
@@ -674,8 +675,10 @@ __device__ __forceinline__ void phase_R(const GsegCtl *ctl, const GsegBufs &B, c
 // emit_row writes one row's survivors and folds them into the next round's per-component minimum.
 // Key = weight bits << 32 | position in the new list (stable compaction keeps list order == edge-index
 // order, so position is the same tie-break as the edge index).
+// CHAIN: round 0, direction E (pixel p -> p + 1): consecutive lanes are consecutive pixels, so every run of equal ends
+// has length one by construction and the row goes straight to the chain form of the minima (warp_chain_min).
 // ------------------------------------------------------------------------------------------------
-template <bool SP, bool FILTER>
+template <bool SP, bool FILTER, bool CHAIN = false>
 __device__ __forceinline__ void emit_row(const GsegBufs &B, int nxt, u32 pos, bool act, u32 a, u32 b, u32 wv,
                                          u32 fa = 0xFFFFFFFFu, u32 fb = 0xFFFFFFFFu, u32 *sfilter = nullptr) {
     u32 kb = wv;
@@ -687,24 +690,8 @@ __device__ __forceinline__ void emit_row(const GsegBufs &B, int nxt, u32 pos, bo
         if (SP) kb = __float_as_uint(__fmul_rn(__uint_as_float(wv), mean_dist_m(B.cmean[nxt], a, b)));
     }
 #ifndef GSEG_EXP_NOMIN
-    warp_run_min2<FILTER, FILTER ? 32 : RUNWIN>(B.best[nxt], a, b, kb, pos, act, fa, fb, sfilter);
-#endif
-}
-
-// Round 0, direction E (pixel p -> p + 1): consecutive lanes are consecutive pixels, so every run of equal ends has length
-// one by construction and the row goes straight to the chain form of the minima (warp_chain_min).
-template <bool SP>
-__device__ __forceinline__ void emit_row_east(const GsegBufs &B, int nxt, u32 pos, bool act, u32 a, u32 b, u32 wv) {
-    u32 kb = wv;
-    if (act) {
-#ifndef GSEG_EXP_NOSTORE
-        B.eab[nxt][pos] = make_uint2(a, b);
-        B.ew[nxt][pos] = wv;
-#endif
-        if (SP) kb = __float_as_uint(__fmul_rn(__uint_as_float(wv), mean_dist_m(B.cmean[nxt], a, b)));
-    }
-#ifndef GSEG_EXP_NOMIN
-    warp_chain_min(B.best[nxt], a, b, kb, pos, act, __ballot_sync(0xFFFFFFFFu, act));
+    if constexpr (CHAIN) warp_chain_min(B.best[nxt], a, b, kb, pos, act, __ballot_sync(0xFFFFFFFFu, act));
+    else warp_run_min2<FILTER, FILTER ? 32 : RUNWIN>(B.best[nxt], a, b, kb, pos, act, fa, fb, sfilter);
 #endif
 }
 
@@ -739,7 +726,7 @@ __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.
 #define R0_BUF (3 * R0_STREAM)                           // one page: a ends, b ends, weights
 #define R0_SMEM ((NT / 32) * (2 * R0_BUF * 4 + 16))      // bytes per block: two page buffers and two mbarriers per warp
 struct R0Page {
-    int d, off; // direction, pixel offset of the b end
+    int d, dx, dy, off; // direction, its step in x and y, pixel offset of the b end (dy w + dx)
     u32 p0;     // first pixel of the page
     u32 src[3]; // 16-byte aligned first word of each stream: map (a), map (b), wgrid
     u32 n[3];   // words to copy (multiple of 4, may be 0)
@@ -747,7 +734,9 @@ struct R0Page {
 __device__ __forceinline__ R0Page r0_page(u32 tile, u32 tpd, u32 V, int w) {
     R0Page pg;
     pg.d = (int)(tile / tpd);
-    pg.off = pg.d == 0 ? 1 : pg.d == 1 ? w : pg.d == 2 ? w + 1 : 1 - w;
+    pg.dx = pg.d == 1 ? 0 : 1;
+    pg.dy = pg.d == 0 ? 0 : (pg.d == 3 ? -1 : 1);
+    pg.off = pg.dy * w + pg.dx;
     pg.p0 = (tile - (u32)pg.d * tpd) * GSEG_PAGE;
     const long long end = min((long long)pg.p0 + GSEG_PAGE, (long long)V);
     const long long lo[3] = {pg.p0, max((long long)pg.p0 + pg.off, 0LL), (long long)pg.d * V + pg.p0};
@@ -805,76 +794,45 @@ __global__ void __launch_bounds__(NT, GSEG_LB_EDGES) k_r0_edges(GsegCtl *ctl, Gs
     u32 esum = 0;
     if (blockIdx.x == 0 && threadIdx.x == 0) ctl->ticketC = 0;
     u32 tile = blockIdx.x * (NT / 32) + wid;
-    if constexpr (!STAGED) {
-        for (; tile < ntiles; tile += nw) {
-            const int d = (int)(tile / tpd);
-            const int dx = d == 1 ? 0 : 1, dy = d == 0 ? 0 : (d == 3 ? -1 : 1);
-            const int off = dy * w + dx;
-            const u32 p0 = (tile - (u32)d * tpd) * GSEG_PAGE + lane;
-            u32 a[ROWS], b[ROWS], m[ROWS], wv[ROWS];
-            const u32 *wg = wgrid + (size_t)d * V + p0;
-            int y = (int)(p0 / (u32)w), x = (int)(p0 - (u32)y * (u32)w);
-#pragma unroll
-            for (int j = 0; j < ROWS; ++j) {
-                const u32 p = p0 + 32u * j;
-                bool keep = false;
-                a[j] = b[j] = wv[j] = 0u;
-                if (p < V && x + dx < w && y + dy < h && y + dy >= 0) {
-                    a[j] = map[p];
-                    b[j] = map[(u32)((int)p + off)];
-                    wv[j] = wg[32 * j]; // with the ids, not row by row between the emits: one round trip per page
-                    keep = a[j] != b[j];
-                }
-                m[j] = __ballot_sync(0xFFFFFFFFu, keep);
-                x += 32;
-                while (x >= w) { x -= w; ++y; }
-            }
-            u32 total = 0;
-#pragma unroll
-            for (int j = 0; j < ROWS; ++j) total += __popc(m[j]);
-            if (lane == 0) { B.pcnt[1][tile] = total; B.poff[1][tile] = tile * GSEG_PAGE; }
-            GSEG_CHK(ctl, (unsigned long long)tile * GSEG_PAGE + total <= ctl->p.edge_slots, 4);
-            esum += total;
-            u32 rowoff = tile * GSEG_PAGE;
-#pragma unroll
-            for (int j = 0; j < ROWS; ++j) {
-                if (m[j] == 0u) continue; // warp-uniform
-                const bool act = (m[j] >> lane) & 1u;
-                if (d == 0) emit_row_east<SP>(B, 1, rowoff + __popc(m[j] & lt), act, a[j], b[j], wv[j]);
-                else emit_row<SP, false>(B, 1, rowoff + __popc(m[j] & lt), act, a[j], b[j], wv[j]);
-                rowoff += __popc(m[j]);
-            }
+    if constexpr (STAGED) {
+        if (lane == 0) {
+            mbar_init(bar);
+            mbar_init(bar + 1);
+            if (tile < ntiles) stage(tile, 0u);
         }
-    } else {
-    if (lane == 0) {
-        mbar_init(bar);
-        mbar_init(bar + 1);
-        if (tile < ntiles) stage(tile, 0u);
+        __syncwarp();
     }
-    __syncwarp();
     for (u32 it = 0; tile < ntiles; tile += nw, ++it) {
         const u32 k = it & 1u;
-        __syncwarp(); // every lane has finished reading buffer k ^ 1 (page tile - nw): refill it
-        if (lane == 0 && tile + nw < ntiles) stage(tile + nw, k ^ 1u);
+        if constexpr (STAGED) {
+            __syncwarp(); // every lane has finished reading buffer k ^ 1 (page tile - nw): refill it
+            if (lane == 0 && tile + nw < ntiles) stage(tile + nw, k ^ 1u);
+        }
         const R0Page pg = r0_page(tile, tpd, V, w);
-        const int d = pg.d, off = pg.off;
-        const int dx = d == 1 ? 0 : 1, dy = d == 0 ? 0 : (d == 3 ? -1 : 1);
+        const int d = pg.d, dx = pg.dx, dy = pg.dy;
         const u32 p0 = pg.p0 + lane;
-        const u32 *sa = buf + k * R0_BUF + lane;                                          // map[p0 + i]
-        const u32 *sb = buf + k * R0_BUF + R0_STREAM + (int)(pg.p0 + off - pg.src[1]) + lane; // map[p0 + off + i]
-        const u32 *sw = buf + k * R0_BUF + 2 * R0_STREAM + (d * V + pg.p0 - pg.src[2]) + lane; // wgrid[d V + p0 + i]
-        // rows are read from the buffer twice (for the survivor ballots, then for the emits) instead of being
-        // held in registers across the emits: 8 rows x (a, b, w) registers less, no spills
-        u32 m[ROWS], live = 0u; // live bit j: row j's edge exists (inside the image)
+        const u32 *sa = buf + k * R0_BUF + lane;                                               // map[p0 + i]
+        const u32 *sb = buf + k * R0_BUF + R0_STREAM + (int)(pg.p0 + pg.off - pg.src[1]) + lane; // map[p0 + off + i]
+        const u32 *sw = buf + k * R0_BUF + 2 * R0_STREAM + (d * V + pg.p0 - pg.src[2]) + lane;  // wgrid[d V + p0 + i]
+        const u32 *wg = wgrid + (size_t)d * V + p0;
+        // Row j's (a, b, w) is (sa, sb, sw)[32 j] in buffer k or (map[p], map[p + off], wg[32 j]) in global memory.  The
+        // register-load body holds the rows in a[], b[], wv[] from the ballots to the emits.  The staged body reads
+        // them from the buffer twice (for the survivor ballots, then for the emits): 8 rows x (a, b, w) registers less, no spills.
+        // The choice is spelled out at each read: a row-source lambda costs the staged body 3 registers (63 instead of 60).
+        u32 a[ROWS], b[ROWS], wv[ROWS], m[ROWS], live = 0u; // live bit j: row j's edge exists (inside the image)
         int y = (int)(p0 / (u32)w), x = (int)(p0 - (u32)y * (u32)w);
-        mbar_wait(bar + k, (it >> 1) & 1u);
+        if constexpr (STAGED) mbar_wait(bar + k, (it >> 1) & 1u);
 #pragma unroll
         for (int j = 0; j < ROWS; ++j) {
             const u32 p = p0 + 32u * j;
             bool keep = false;
+            a[j] = b[j] = wv[j] = 0u;
             if (p < V && x + dx < w && y + dy < h && y + dy >= 0) {
                 live |= 1u << j;
-                keep = sa[32 * j] != sb[32 * j];
+                a[j] = STAGED ? sa[32 * j] : map[p];
+                b[j] = STAGED ? sb[32 * j] : map[(u32)((int)p + pg.off)];
+                if constexpr (!STAGED) wv[j] = wg[32 * j]; // with the ids, not row by row between the emits: one round trip per page
+                keep = a[j] != b[j];
             }
             m[j] = __ballot_sync(0xFFFFFFFFu, keep);
             x += 32;
@@ -891,12 +849,12 @@ __global__ void __launch_bounds__(NT, GSEG_LB_EDGES) k_r0_edges(GsegCtl *ctl, Gs
         for (int j = 0; j < ROWS; ++j) {
             if (m[j] == 0u) continue; // warp-uniform
             const bool act = (m[j] >> lane) & 1u, in = (live >> j) & 1u;
-            const u32 a = in ? sa[32 * j] : 0u, b = in ? sb[32 * j] : 0u, wv = in ? sw[32 * j] : 0u;
-            if (d == 0) emit_row_east<SP>(B, 1, rowoff + __popc(m[j] & lt), act, a, b, wv);
-            else emit_row<SP, false>(B, 1, rowoff + __popc(m[j] & lt), act, a, b, wv);
+            const u32 ra = !STAGED ? a[j] : in ? sa[32 * j] : 0u, rb = !STAGED ? b[j] : in ? sb[32 * j] : 0u,
+                      rw = !STAGED ? wv[j] : in ? sw[32 * j] : 0u;
+            if (d == 0) emit_row<SP, false, true>(B, 1, rowoff + __popc(m[j] & lt), act, ra, rb, rw);
+            else emit_row<SP, false>(B, 1, rowoff + __popc(m[j] & lt), act, ra, rb, rw);
             rowoff += __popc(m[j]);
         }
-    }
     }
     if (lane == 0 && esum) atomicAdd(&ctl->Eacc[0], esum);
     RoundState s0 = st;
@@ -1149,38 +1107,29 @@ __device__ __forceinline__ void phase_E_rows(GsegCtl *ctl, const GsegBufs &B, co
             }
             u32 rowoff = out_base + written + before;
             GSEG_CHK(ctl, (unsigned long long)out_base + written + total <= ctl->p.edge_slots, 9);
-            if (filter && staged) {
+            u32 fa[RW] = {}, fb[RW] = {}; // filter, not staged: the weights of the current minima of both ends
+            auto emit = [&](auto filt, u32 *sfilter) {
 #pragma unroll
                 for (int j = 0; j < RW; ++j) {
                     if (m[j] == 0u) continue; // warp-uniform
                     const bool act = (m[j] >> lane) & 1u;
-                    emit_row<SP, true>(B, nxt, rowoff + __popc(m[j] & lt), act, a[j], b[j], wv[j], 0u, 0u, s_bhi);
+                    emit_row<SP, decltype(filt)::value>(B, nxt, rowoff + __popc(m[j] & lt), act, a[j], b[j], wv[j], fa[j], fb[j], sfilter);
                     rowoff += __popc(m[j]);
                 }
+            };
+            if (filter && staged) {
+                emit(std::true_type{}, s_bhi);
             } else if (filter) {
-                // weights of the current minima of both ends, for all rows at once (one round trip)
-                u32 fa[RW], fb[RW];
+                // for all rows at once, ahead of the emits (one round trip)
                 const u32 *bhi = reinterpret_cast<const u32 *>(B.best[nxt]) + 1; // high word = weight bits
 #pragma unroll
                 for (int j = 0; j < RW; ++j) {
                     fa[j] = fb[j] = 0xFFFFFFFFu;
                     if ((m[j] >> lane) & 1u) { fa[j] = ld_relaxed_u32(bhi + 2 * (size_t)a[j]); fb[j] = ld_relaxed_u32(bhi + 2 * (size_t)b[j]); }
                 }
-#pragma unroll
-                for (int j = 0; j < RW; ++j) {
-                    if (m[j] == 0u) continue; // warp-uniform
-                    const bool act = (m[j] >> lane) & 1u;
-                    emit_row<SP, true>(B, nxt, rowoff + __popc(m[j] & lt), act, a[j], b[j], wv[j], fa[j], fb[j]);
-                    rowoff += __popc(m[j]);
-                }
+                emit(std::true_type{}, nullptr);
             } else {
-#pragma unroll
-                for (int j = 0; j < RW; ++j) {
-                    if (m[j] == 0u) continue; // warp-uniform
-                    const bool act = (m[j] >> lane) & 1u;
-                    emit_row<SP, false>(B, nxt, rowoff + __popc(m[j] & lt), act, a[j], b[j], wv[j]);
-                    rowoff += __popc(m[j]);
-                }
+                emit(std::false_type{}, nullptr);
             }
             written += total;
         }
@@ -1364,24 +1313,26 @@ __global__ void __launch_bounds__(1024) k_compact_keep(GsegCtl *ctl, const uint2
         __syncthreads();
     }
 }
-// Import: dense pages of GSEG_PAGE slots over a caller-supplied edge list (slot = list position = the
-// tie-break) and the per-component minimum of round 1.
-__global__ void __launch_bounds__(NT) k_graph_init(GsegBufs B, u32 E, u32 P) {
+// Dense list of E edges on buffer side `side`: its P pages of GSEG_PAGE slots (slot = list position = the
+// tie-break) and the per-component minimum of the round that reads it.  One warp per page.
+template <int side>
+__device__ __forceinline__ void seed_dense_pages(const GsegBufs &B, u32 E, u32 P) {
     const int lane = threadIdx.x & 31;
     for (u32 g = blockIdx.x * (NT / 32) + (threadIdx.x >> 5); g < P; g += gridDim.x * (NT / 32)) {
-        if (lane == 0) { B.pcnt[1][g] = min(GSEG_PAGE, E - g * GSEG_PAGE); B.poff[1][g] = g * GSEG_PAGE; }
+        if (lane == 0) { B.pcnt[side][g] = min(GSEG_PAGE, E - g * GSEG_PAGE); B.poff[side][g] = g * GSEG_PAGE; }
 #pragma unroll
         for (int j = 0; j < (int)(GSEG_PAGE / 32); ++j) {
             const u32 e = g * GSEG_PAGE + 32u * j + lane;
             const bool act = e < E;
             uint2 ab = make_uint2(0u, 0u);
             u32 wv = 0u;
-            if (act) { ab = B.eab[1][e]; wv = B.ew[1][e]; }
-            warp_run_min<false, 32>(B.best[1], ab.x, wv, e, act, 0xFFFFFFFFu);
-            warp_run_min<false, 32>(B.best[1], ab.y, wv, e, act, 0xFFFFFFFFu);
+            if (act) { ab = B.eab[side][e]; wv = B.ew[side][e]; }
+            warp_run_min2<false, 32>(B.best[side], ab.x, ab.y, wv, e, act, 0xFFFFFFFFu, 0xFFFFFFFFu);
         }
     }
 }
+// Import: pages over a caller-supplied edge list and the per-component minimum of round 1.
+__global__ void __launch_bounds__(NT) k_graph_init(GsegBufs B, u32 E, u32 P) { seed_dense_pages<1>(B, E, P); }
 
 // ---- tiled schedule on the device (BASELINE.json configs[4]; DESIGN.md "Tiled schedule") ---------------
 // Strip record (32-bit words, device memory): header[8] = {magic, nV, nE, w, 0...} | attr uint2[nV] (size, Int bits)
